@@ -6,6 +6,12 @@ per GPU-job, rho sweep), on N B200s, next to the reference's own CPU implementat
     python bench.py --gpus N --steps K --warmup W            # this implementation
     python bench.py --impl reference --steps K --warmup W     # the UNMODIFIED reference (oracle/_ref, see oracle/make_ref.py)
     python bench.py --impl port --steps K --warmup W          # the oracle port (numpy restatement) on all host cores
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   # also writes the last timed step's outputs
+
+`--dump-outputs DIR` writes what the last timed step returned, so that two builds can be compared output for
+output (same arguments -> same plans, coefficients and Philox streams): DIR/acc.npy and DIR/shift.npy, the
+all-reduced accumulator of mcre_irc_mainsim and its pilot shifts (float64, one entry per slot), and DIR/cva.npy,
+[CVA, Monte Carlo error] finished from them the way SimulationController.run_simulation() does.
 
 A "step" is one full main-simulation pass (all paths x 240 sub-steps, one rho of the sweep)
 with the plan and regression coefficients resident in HBM.  `e2e` times the public API
@@ -257,7 +263,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true", help="kernel tuning runs: skip the end-to-end leg")
     ap.add_argument("--ref-paths-log2", type=int, default=17, help="main-simulation paths per step of the reference arm")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference_arm(args)
     if args.impl == "port":
@@ -301,7 +310,7 @@ def main():
         arr, ptr = B.as_dp(coef)
         B.check(L.mcre_irc_set_coefficients(plan, ptr, RT.stream_ptr()))
         torch.cuda.synchronize()
-        plans.append((plan, keep, sc))
+        plans.append((plan, keep, sc, info))
     begin, count = RT.shard_range(n_total, CHUNK_PATHS)
     slots = L.mcre_irc_main_slots(plans[0][0])
     acc = torch.zeros(slots, dtype=torch.float64, device=dev)
@@ -339,6 +348,16 @@ def main():
     barrier()
     launches = B.launch_count() - launches0
     sampler.stop_flag = True
+    if args.dump_outputs and rank == 0:
+        from mcre.finish import irc_raw_to_neutral
+        info = plans[(args.warmup + args.steps - 1) % len(plans)][3]
+        acc_h, shift_h = total.cpu().numpy(), shift.cpu().numpy()
+        rows = info["n_metric"] + 1
+        res = irc_raw_to_neutral(acc_h.reshape(rows, -1), shift_h.reshape(rows, -1), n_total, 0, info["n_metric"],
+                                 info["acc"])
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in (("acc", acc_h), ("shift", shift_h), ("cva", np.array(res["cva"][0], dtype=np.float64))):
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), arr)
     ms_total = ev[0].elapsed_time(ev[-1])
     t = torch.tensor([ms_total], dtype=torch.float64, device=dev)
     if world > 1:
@@ -448,7 +467,7 @@ def main():
                 "clocks": sampler.summary(), "e2e": e2e, "gpu_launches": int(launches), "roofline": roofline,
                 "cpu_baseline": cpu, "parity_check": parity}
         print(json.dumps(line))
-    for plan, _, _ in plans:
+    for plan, *_ in plans:
         L.mcre_irc_destroy(plan)
     if world > 1:
         dist.destroy_process_group()
