@@ -445,7 +445,12 @@ int mcre_eq_presim(mcre_eq_plan *plan, const mcre_rng *rng, const mcre_shard *sh
  *    cashflows with respect to the parameters of the product's asset), which feed mcre_lsm_step_tangents;
  *  - mcre_eq_set_exposure_coef_tangents: host xp_tan [n_expo][n_prod][3][nt], d(c0, c1, c2)/d(lane parameters) from the
  *    differentiated normal equations (the reference keeps torch.linalg.lstsq in the autograd graph,
- *    controller.py:368-383); copied to the device. */
+ *    controller.py:368-383); copied to the device;
+ *  - mcre_eq_set_exercise_exposure_coef_tangents: the same for exercise products (exposure type 3): host
+ *    [n_expo][n_prod][MCRE_LSM_MAX_RIGHTS][3][nt], d(c0, c1, c2)/d(lane parameters) of the continuation value of state
+ *    s = rights left at row s - 1 (from the tangent backward induction, mcre_lsm_step_states_tangents); rows of other
+ *    products are ignored.  The exposure of state s is (c0 + u (c1 + u c2)) / N(t) on duals, 0 in state 0; the state
+ *    itself carries no tangent.  Copied to the device. */
 /* Hybrid ModelConfig of Black-Scholes market models + the CIR++ credit model of a counterparty (the reference's
  * tests/exposure_tests/cva_perfprmance_large_netting_set.py): the fused equity kernel also steps the intensity
  * (cirpp.py:155-198, Euler with full truncation or the deterministic mode) on the noise column `noise_col` of the joint
@@ -480,6 +485,7 @@ int mcre_eq_cva_paths(const double *d_unsec, const double *d_w, int64_t n_paths,
 int mcre_eq_presim_tangents(mcre_eq_plan *plan, const mcre_rng *rng, const mcre_shard *shard, double *d_partial,
                             double *d_shift, double *d_x, float *d_cf, double *d_dx, double *d_dcf, void *stream);
 int mcre_eq_set_exposure_coef_tangents(mcre_eq_plan *plan, const double *xp_tan);
+int mcre_eq_set_exercise_exposure_coef_tangents(mcre_eq_plan *plan, const double *tan);
 
 /* ================================================================================
  * Longstaff-Schwartz backward induction on spilled pre-simulation arrays: one call per
@@ -554,6 +560,18 @@ int mcre_lsm_step_tangents(int32_t nt, const double *d_xk, const double *d_nk, c
                            const double *d_dni, const double *d_dimm, const double *coef_i, double shift_i, double scale_i,
                            const float *d_value, double *d_dvalue, int64_t n, int32_t chunk_paths, double *d_partial,
                            double *d_tmoments, void *stream);
+/* The same for 1..6 exercise rights, called after mcre_lsm_step_states for the same regression date (n_rights = 1:
+ * exactly mcre_lsm_step_tangents).  Recomputes every state's decision ex_s = imm_i + cont(s-1) > cont(s) with the
+ * expressions of the value step and updates the running tangents d_dvalue [n_rights][nt][n] from their values before
+ * the update:  dV_s <- ex_s ? (dimm_i - (imm_i / N_i) dN_i) / N_i + dV_{s-1} : dV_s  (dV_0 = 0).  coef_i: host
+ * [n_rights][3] or NULL; d_value: the value step's [n_rights][n].  d_tmoments [nt][4 + 5 n_rights]: sum u^m du
+ * (m = 0..3), then per state s at 4 + 5 s: sum dY, u dY, u^2 dY, du Y, 2 u du Y with Y = N_k V_s. */
+int mcre_lsm_step_states_tangents(int32_t n_rights, int32_t nt, const double *d_xk, const double *d_nk,
+                                  const double *d_dxk, const double *d_dnk, double shift_k, double scale_k,
+                                  const double *d_xi, const double *d_ni, const double *d_imm, const double *d_dni,
+                                  const double *d_dimm, const double *coef_i, double shift_i, double scale_i,
+                                  const float *d_value, double *d_dvalue, int64_t n, int32_t chunk_paths,
+                                  double *d_partial, double *d_tmoments, void *stream);
 
 /* LSM pre-simulation arrays of an exercise product on equity underlyings, gathered date-major from
  * materialised pre-simulation paths (mcre_generate_paths with seed 42; the pre-simulation is a small
@@ -567,6 +585,15 @@ int mcre_lsm_prepare_equity(const double *d_paths, int64_t n_paths, int32_t n_da
                             int32_t n_under, const int32_t *under_col, const double *under_w,
                             const int32_t *under_is_log, double strike, const double *ex_strike, double sign,
                             double *d_x, double *d_n, double *d_imm, void *stream);
+/* Pathwise tangents of those arrays (single-asset exercise products), from the tangent spill of the pre-simulation
+ * d_dx [n_rows][n_assets][nt][n_paths] (mcre_eq_presim_tangents on a plan whose exposure dates are the spill dates):
+ * d_dxs [n_reg][nt][n] = the spill row reg_row[k] of asset x_asset; d_dnum [n_reg][nt][n] = reg_dnum[k] in parameter
+ * rate_slot, 0 elsewhere (the numeraire is deterministic); d_dimm [n_ex][nt][n] = sign * 1{imm > 0} * the spill row
+ * ex_row[i] of asset u_asset.  d_imm: the value arrays of mcre_lsm_prepare_equity.  Host index tables. */
+int mcre_lsm_prepare_equity_tangents(const double *d_dx, int64_t n_paths, int32_t n_assets, int32_t nt, int32_t n_reg,
+                                     const int32_t *reg_row, const double *reg_dnum, int32_t rate_slot, int32_t x_asset,
+                                     int32_t n_ex, const int32_t *ex_row, int32_t u_asset, double sign,
+                                     const double *d_imm, double *d_dxs, double *d_dnum, double *d_dimm, void *stream);
 
 /* ================================================================================
  * Exact order statistics per row (PFE), replaces torch.sort + index in

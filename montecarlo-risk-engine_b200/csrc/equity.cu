@@ -81,6 +81,9 @@ struct EqDev {
   // and the tangent spill of the pre-simulation pass (mcre_eq_presim_tangents): ps_dx [n_expo][A][nt][n_paths],
   // ps_dcf [n_prod][nt][n_paths] (f64: the reference's float32 rounding touches values only under autograd's chain)
   const double *xp_tan;
+  // ... and of the continuation values of exercise products (exposure type 3), per state s = rights left at row s - 1:
+  // [n_expo][n_prod][EQ_MAX_RIGHTS][3 coefficients][nt] (mcre_eq_set_exercise_exposure_coef_tangents)
+  const double *xp_ex_tan;
   // per exposure date the products whose record carries an exposure (type != 0), ascending: xact[xact_off[e] .. xact_off[e+1])
   // (built by mcre_eq_create from xp; matured products and the other launches' products are never visited)
   const int *xact_off, *xact;
@@ -102,6 +105,7 @@ constexpr int EQ_PF = 8;     // exposure records prefetched ahead of the walk (m
 __device__ __forceinline__ void prefetch_l1(const void *p) { asm volatile("prefetch.global.L1 [%0];" ::"l"(p)); }
 constexpr int EQ_EVD = 32;  // doubles per event record ([16 + 3 (st - 2)]: continuation coefficients of states 2..6) (exercise events: see mcre_eq_desc.ev_data)
 constexpr int EQ_MAX_LAG = 4;
+constexpr int EQ_MAX_RIGHTS = MCRE_LSM_MAX_RIGHTS;
 constexpr int EQ_SPNZ = 8;   // non-zeros kept per sparse correlation row
 
 enum { EQ_EUROPEAN = MCRE_EQ_EUROPEAN, EQ_BINARY = MCRE_EQ_BINARY, EQ_BASKET = MCRE_EQ_BASKET, EQ_ASIAN = MCRE_EQ_ASIAN,
@@ -356,6 +360,30 @@ __global__ void __launch_bounds__(128, (NT == 0 ? 4 : 2)) eq_main_kernel(EqDev P
                   const int setq = (int)__ldg(pr + 1);
 #pragma unroll
                   for (int s = 0; s < NS; ++s) if (s == setq) expo[s] = expo[s] + totq;
+                  continue;
+                }
+                if (xtype == 3 && P.xp_ex_tan) {
+                  // exercise products: the quadratic of the current state on duals (coefficients and their tangents
+                  // selected by the state, which itself carries none: the reference gathers coefficients by state)
+                  XR ve = RealTraits<XR>::zero();
+                  if (xw != 0.0 && st > 0) {
+                    const R ue = (spot_now() - __ldg(op + 5)) * __ldg(op + 6);
+                    const double *cv = st == 1 ? op + 1 : op + 16 + 3 * (st - 2);
+                    const int o1 = st == 1 ? 2 : 1;     // state 1 keeps 1 / N(t) between c0 and c1
+                    R e0 = T::lift(__ldg(cv)), e1 = T::lift(__ldg(cv + o1)), e2 = T::lift(__ldg(cv + o1 + 1));
+                    const double *ct = P.xp_ex_tan + (((size_t)xe * P.n_prod + pi) * EQ_MAX_RIGHTS + (st - 1)) * 3 * NT;
+#pragma unroll
+                    for (int k = 0; k < NT; ++k) {
+                      e0.d[k] = __ldg(ct + k); e1.d[k] = __ldg(ct + NT + k); e2.d[k] = __ldg(ct + 2 * NT + k);
+                    }
+                    const R poly = e0 + ue * (e1 + ue * e2);
+                    ve = poly * __ldg(op + 2);
+                    ve.d[2] += val(poly) * __ldg(op + 7);
+                  }
+                  const XR tote = r_with_value(ve, group_sum(val(ve), base, A));
+                  const int sete = (int)__ldg(pr + 1);
+#pragma unroll
+                  for (int s = 0; s < NS; ++s) if (s == sete) expo[s] = expo[s] + tote;
                   continue;
                 }
               }
@@ -857,8 +885,10 @@ struct mcre_eq_plan {
   DevArray<int> date_expo, date_metric, set_flags, set_lag, sp_src, xact_off, xact;
   DevArray<double> xp, set_threshold, sp_coef;
   double *xp_tan = nullptr;   // own allocation (set after mcre_eq_create)
+  double *xp_ex_tan = nullptr;   // own allocation (mcre_eq_set_exercise_exposure_coef_tangents)
   double *credit = nullptr;   // own allocation (mcre_eq_set_credit): step_cir, cir_row, cva_coef, set_cva
   bool has_proxy = false;     // some exposure is a regression proxy (type 2)
+  bool has_exercise_expo = false;   // some exposure is an exercise product's continuation value (type 3)
 };
 
 extern "C" int mcre_eq_create(const mcre_eq_desc *c, mcre_eq_plan **out) {
@@ -877,8 +907,8 @@ extern "C" int mcre_eq_create(const mcre_eq_desc *c, mcre_eq_plan **out) {
     if (!eq_kind_has_exposure_tangents(c->kind))
       return fail(-4, "eq: sensitivities of exposure profiles need a Black-Scholes or Heston model%s", "");
     for (size_t i = 0; i < (size_t)c->n_expo * c->n_prod; ++i)
-      if (c->xp[i * EQ_XP] > 2.0)
-        return fail(-4, "eq: sensitivities of the exposures of exercise products are not implemented%s", "");
+      if (c->xp[i * EQ_XP] > 3.0)
+        return fail(-4, "eq: unknown exposure type%s", "");
   }
   if (c->corr_mode == 1 && (c->n_assets != 1 || c->noise_dim != 2))
     return fail(-1, "eq: dual Cholesky needs one asset with two noise sources%s", "");
@@ -896,7 +926,10 @@ extern "C" int mcre_eq_create(const mcre_eq_desc *c, mcre_eq_plan **out) {
   mcre_eq_plan *p = new mcre_eq_plan();
   ArenaScope arena_scope(&p->arena);
   p->nt = c->nt;
-  for (size_t i = 0; c->n_expo > 0 && i < (size_t)c->n_expo * c->n_prod; ++i) p->has_proxy = p->has_proxy || c->xp[i * EQ_XP] == 2.0;
+  for (size_t i = 0; c->n_expo > 0 && i < (size_t)c->n_expo * c->n_prod; ++i) {
+    p->has_proxy = p->has_proxy || c->xp[i * EQ_XP] == 2.0;
+    p->has_exercise_expo = p->has_exercise_expo || c->xp[i * EQ_XP] == 3.0;
+  }
   const int A = c->n_assets, d = c->noise_dim, n_ev = c->date_ev_off[c->n_dates];
   int rc = 0;
 #define UP(field, host, count) if (!rc) rc = p->field.upload(host, (size_t)(count))
@@ -954,7 +987,7 @@ extern "C" int mcre_eq_create(const mcre_eq_desc *c, mcre_eq_plan **out) {
   if (rc) { mcre_eq_destroy(p); return rc; }
   EqDev &D = p->d;
   D.sp_n = sp_n; D.sp_coef = p->sp_coef.p; D.sp_src = p->sp_src.p; D.n_sub_total = c->n_sub;
-  D.xp_tan = nullptr; D.ps_dx = nullptr; D.ps_dcf = nullptr;
+  D.xp_tan = nullptr; D.xp_ex_tan = nullptr; D.ps_dx = nullptr; D.ps_dcf = nullptr;
   D.has_cir = 0; D.cir_det = 0; D.cir_col = 0; D.cir_kappa = D.cir_theta = D.cir_sigma = D.cir_y0 = D.lgd = 0.0;
   D.step_cir = D.cir_row = D.cva_coef = nullptr; D.set_cva = nullptr; D.cva_w = nullptr;
   D.ps_x = nullptr; D.ps_cf = nullptr; D.pv_accum = nullptr; D.bridge_u = nullptr; D.bridge_stride = 0; D.expo_accum = nullptr; D.expo_accum_tan = nullptr;
@@ -989,6 +1022,7 @@ extern "C" void mcre_eq_destroy(mcre_eq_plan *p) {
   p->xact_off.release(); p->xact.release();
   p->arena.release();
   if (p->xp_tan) cudaFree(p->xp_tan);
+  if (p->xp_ex_tan) cudaFree(p->xp_ex_tan);
   if (p->credit) cudaFree(p->credit);
   delete p;
 }
@@ -1001,6 +1035,17 @@ extern "C" int mcre_eq_set_exposure_coef_tangents(mcre_eq_plan *p, const double 
   if (!p->xp_tan) MCRE_CUDA(cudaMalloc((void **)&p->xp_tan, n * sizeof(double)));
   MCRE_CUDA(cudaMemcpy(p->xp_tan, xp_tan, n * sizeof(double), cudaMemcpyHostToDevice));
   p->d.xp_tan = p->xp_tan;
+  return 0;
+}
+
+extern "C" int mcre_eq_set_exercise_exposure_coef_tangents(mcre_eq_plan *p, const double *tan) {
+  if (!p || !tan) return fail(-1, "null argument%s", "");
+  if (p->nt <= 0 || !eq_kind_has_exposure_tangents(p->d.kind) || p->d.n_expo <= 0)
+    return fail(-4, "eq: coefficient tangents need a Black-Scholes / Heston plan with tangents and exposure dates%s", "");
+  const size_t n = (size_t)p->d.n_expo * p->d.n_prod * EQ_MAX_RIGHTS * 3 * p->nt;
+  if (!p->xp_ex_tan) MCRE_CUDA(cudaMalloc((void **)&p->xp_ex_tan, n * sizeof(double)));
+  MCRE_CUDA(cudaMemcpy(p->xp_ex_tan, tan, n * sizeof(double), cudaMemcpyHostToDevice));
+  p->d.xp_ex_tan = p->xp_ex_tan;
   return 0;
 }
 
@@ -1113,6 +1158,9 @@ extern "C" int mcre_eq_mainsim(mcre_eq_plan *p, const mcre_rng *rng, const mcre_
     return fail(-1, "spill requested but d_spill is null%s", "");
   if (p->nt > 0 && p->has_proxy && !p->d.xp_tan && !p->d.ps_x)
     return fail(-1, "eq: plan with tangents and regression-proxy exposures: call mcre_eq_set_exposure_coef_tangents first%s", "");
+  if (p->nt > 0 && p->has_exercise_expo && !p->d.xp_ex_tan && !p->d.ps_x)
+    return fail(-1, "eq: plan with tangents and exposures of exercise products: call "
+                    "mcre_eq_set_exercise_exposure_coef_tangents first%s", "");
   if (rng->mode == MCRE_RNG_INJECT && p->d.kind == MCRE_EQ_HESTON && p->d.scheme == MCRE_SCHEME_QE && !rng->d_u)
     return fail(-1, "inject mode: QE needs uniforms%s", "");
   RngDev r = make_rng(rng);

@@ -212,6 +212,106 @@ __global__ void __launch_bounds__(256) lsm_moments_batch_kernel(const LsmJob *__
   }
 }
 
+// Tangent companion of lsm_step_kernel<R> for R = 2..6 rights (R = 1: lsm_step_tan_kernel, csrc/irc_tan.cu), run after
+// the value step of the same regression date.  For parameter blockIdx.y it recomputes the exercise decisions with the
+// double expressions of lsm_step_item<R> (so they are the value pass's decisions) and applies them to the running
+// tangents, every state from the values before the update:
+//     dV_s <- ex_s ? d(imm_i / N_i) + dV_{s-1} : dV_s,   d(imm / N) = (dimm - (imm / N) dN) / N,   dV_0 = 0
+// then accumulates the tangent moments of date k with Y_s = N_k V_s, dY_s = dN_k V_s + N_k dV_s (V_s the float32 value
+// the value step has already written): [0..3] sum u^m du (shared by the states), per state s at 4 + 5 s:
+// sum dY, u dY, u^2 dY, du Y, 2 u du Y.  dvalue: [R][nt][n] f64; partial: [chunk][nt][4 + 5 R].
+template <int R>
+__global__ void __launch_bounds__(256) lsm_step_states_tan_kernel(
+    int nt, const double *__restrict__ xk, const double *__restrict__ nk, const double *__restrict__ dxk,
+    const double *__restrict__ dnk, double shift_k, double scale_k, const double *__restrict__ xi,
+    const double *__restrict__ ni, const double *__restrict__ imm, const double *__restrict__ dni,
+    const double *__restrict__ dimm, int has_coef, LsmCoef cf, double shift_i, double scale_i,
+    const float *__restrict__ value, double *__restrict__ dvalue, long long n, int chunk, double *__restrict__ partial) {
+  constexpr int NV = 4 + 5 * R;
+  __shared__ double acc[NV];
+  __shared__ double stage[2 * 8 * NV];
+  const int ip = blockIdx.y;
+  const long long n_chunks = (n + chunk - 1) / chunk;
+  for (long long ch = blockIdx.x; ch < n_chunks; ch += gridDim.x) {
+    if (threadIdx.x < NV) acc[threadIdx.x] = 0.0;
+    __syncthreads();
+    int parity = 0;
+    double vals[NV];
+#pragma unroll
+    for (int j = 0; j < NV; ++j) vals[j] = 0.0;
+    for (int it = 0; it < chunk; it += blockDim.x) {
+      const long long p = ch * chunk + it + threadIdx.x;
+      if (it + (int)threadIdx.x < chunk && p < n) {
+        double dv[R];
+#pragma unroll
+        for (int s = 0; s < R; ++s) dv[s] = dvalue[((size_t)s * nt + ip) * n + p];
+        if (imm) {
+          const double im = imm[p];
+          double cont[R + 1];
+          cont[0] = 0.0;
+          const double ui = has_coef ? (xi[p] - shift_i) * scale_i : 0.0;
+#pragma unroll
+          for (int s = 0; s < R; ++s) cont[s + 1] = has_coef ? cf.c[s][0] + ui * (cf.c[s][1] + ui * cf.c[s][2]) : 0.0;
+          const double inv = 1.0 / ni[p];
+          const double dpay = (dimm[(size_t)ip * n + p] - im * inv * dni[(size_t)ip * n + p]) * inv;
+          double nd[R];
+#pragma unroll
+          for (int s = 0; s < R; ++s) {
+            const bool ex = im + cont[s] > cont[s + 1];
+            nd[s] = ex ? dpay + (s > 0 ? dv[s - 1] : 0.0) : dv[s];
+          }
+#pragma unroll
+          for (int s = 0; s < R; ++s) { dv[s] = nd[s]; dvalue[((size_t)s * nt + ip) * n + p] = nd[s]; }
+        }
+        const double uu = (xk[p] - shift_k) * scale_k, du = dxk[(size_t)ip * n + p] * scale_k;
+        const double u2 = uu * uu, nkp = nk[p], dnkp = dnk[(size_t)ip * n + p];
+        vals[0] += du; vals[1] += uu * du; vals[2] += u2 * du; vals[3] += u2 * uu * du;
+#pragma unroll
+        for (int s = 0; s < R; ++s) {
+          const double V = (double)value[(size_t)s * n + p];
+          const double Y = nkp * V, dY = dnkp * V + nkp * dv[s];
+          double *o = vals + 4 + 5 * s;
+          o[0] += dY; o[1] += uu * dY; o[2] += u2 * dY; o[3] += du * Y; o[4] += 2.0 * uu * du * Y;
+        }
+      }
+    }
+    block_accumulate<NV>(vals, acc, 0, stage, NV, parity);
+    __syncthreads();
+    if (threadIdx.x < NV) partial[((size_t)ch * nt + ip) * NV + threadIdx.x] = acc[threadIdx.x];
+    __syncthreads();
+  }
+}
+
+// Pathwise tangents of the arrays of mcre_lsm_prepare_equity from the tangent spill of the pre-simulation
+// (mcre_eq_presim_tangents, dx [n_rows][A][nt][n]): blockIdx.y = output row (n_reg regression dates, then n_ex exercise
+// dates), threads over paths.
+//   dxs[k][j]  = dx[reg_row[k]][x_asset][j]                 (tangent of the explanatory spot)
+//   dnum[k][j] = j == rate_slot ? reg_dnum[k] : 0           (the deterministic numeraire moves with the rate only)
+//   dimm[i][j] = imm[i] > 0 ? sign dx[ex_row[i]][u_asset][j] : 0
+__global__ void __launch_bounds__(256) lsm_prepare_equity_tan_kernel(const double *__restrict__ dx, long long n, int A, int nt,
+                                                                     int n_reg, const int *__restrict__ reg_row,
+                                                                     const double *__restrict__ reg_dnum, int rate_slot,
+                                                                     int x_asset, int n_ex, const int *__restrict__ ex_row,
+                                                                     int u_asset, double sign, const double *__restrict__ imm,
+                                                                     double *__restrict__ dxs, double *__restrict__ dnum,
+                                                                     double *__restrict__ dimm) {
+  const long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (p >= n) return;
+  const int k = blockIdx.y;
+  if (k < n_reg) {
+    const double *src = dx + ((size_t)reg_row[k] * A + x_asset) * nt * n;
+    for (int j = 0; j < nt; ++j) {
+      dxs[((size_t)k * nt + j) * n + p] = src[(size_t)j * n + p];
+      dnum[((size_t)k * nt + j) * n + p] = j == rate_slot ? reg_dnum[k] : 0.0;
+    }
+  } else {
+    const int i = k - n_reg;
+    const double *src = dx + ((size_t)ex_row[i] * A + u_asset) * nt * n;
+    const bool itm = imm[(size_t)i * n + p] > 0.0;
+    for (int j = 0; j < nt; ++j) dimm[((size_t)i * nt + j) * n + p] = itm ? sign * src[(size_t)j * n + p] : 0.0;
+  }
+}
+
 // Gathers the regression / exercise inputs of an equity exercise product from materialised paths
 // [n_paths][n_dates][state_dim]: blockIdx.y = output row (n_reg regression dates, then n_ex exercise dates), threads
 // over paths: date-major outputs (coalesced writes) and enough threads in flight for books on ~1000 paths (one
@@ -283,6 +383,78 @@ extern "C" int mcre_lsm_prepare_equity(const double *d_paths, int64_t n_paths, i
   rd.release(); ed.release(); uc.release(); ul.release(); rn.release(); uw.release(); xs.release();
   arena.release();
   return rc;
+}
+
+extern "C" int mcre_lsm_prepare_equity_tangents(const double *d_dx, int64_t n_paths, int32_t n_assets, int32_t nt,
+                                                int32_t n_reg, const int32_t *reg_row, const double *reg_dnum,
+                                                int32_t rate_slot, int32_t x_asset, int32_t n_ex, const int32_t *ex_row,
+                                                int32_t u_asset, double sign, const double *d_imm, double *d_dxs,
+                                                double *d_dnum, double *d_dimm, void *stream) {
+  if (!d_dx || !reg_row || !reg_dnum || !ex_row || !d_imm || !d_dxs || !d_dnum || !d_dimm) return fail(-1, "null argument%s", "");
+  if (nt < 1 || n_assets < 1 || x_asset < 0 || x_asset >= n_assets || u_asset < 0 || u_asset >= n_assets)
+    return fail(-1, "lsm prepare tangents: asset or parameter count out of range%s", "");
+  if (n_paths <= 0 || n_reg + n_ex <= 0) return 0;
+  cudaStream_t st = (cudaStream_t)stream;
+  DevArray<int> rr, er;
+  DevArray<double> rd;
+  DevArena arena;
+  ArenaScope arena_scope(&arena);
+  int rc = rr.upload(reg_row, n_reg);
+  if (!rc) rc = er.upload(ex_row, n_ex);
+  if (!rc) rc = rd.upload(reg_dnum, n_reg);
+  if (!rc) rc = arena.commit();
+  if (!rc) {
+    lsm_prepare_equity_tan_kernel<<<dim3((unsigned)((n_paths + 255) / 256), (unsigned)(n_reg + n_ex)), 256, 0, st>>>(
+        d_dx, n_paths, n_assets, nt, n_reg, rr.p, rd.p, rate_slot, x_asset, n_ex, er.p, u_asset, sign, d_imm, d_dxs, d_dnum,
+        d_dimm);
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) rc = cuda_fail(e, "kernel launch");
+    else cudaStreamSynchronize(st);   // the temporary index tables are freed below
+  }
+  rr.release(); er.release(); rd.release();
+  arena.release();
+  return rc;
+}
+
+extern "C" int mcre_lsm_step_states_tangents(int32_t n_rights, int32_t nt, const double *d_xk, const double *d_nk,
+                                             const double *d_dxk, const double *d_dnk, double shift_k, double scale_k,
+                                             const double *d_xi, const double *d_ni, const double *d_imm,
+                                             const double *d_dni, const double *d_dimm, const double *coef_i,
+                                             double shift_i, double scale_i, const float *d_value, double *d_dvalue,
+                                             int64_t n, int32_t chunk_paths, double *d_partial, double *d_tmoments,
+                                             void *stream) {
+  if (n_rights < 1 || n_rights > LSM_MAX_RIGHTS) return fail(-3, "lsm: 1..6 exercise rights are supported%s", "");
+  if (n_rights == 1)   // one right: the rate family's kernel, bit for bit
+    return mcre_lsm_step_tangents(nt, d_xk, d_nk, d_dxk, d_dnk, shift_k, scale_k, d_xi, d_ni, d_imm, d_dni, d_dimm, coef_i,
+                                  shift_i, scale_i, d_value, d_dvalue, n, chunk_paths, d_partial, d_tmoments, stream);
+  if (!d_xk || !d_nk || !d_dxk || !d_dnk || !d_value || !d_dvalue || !d_partial || !d_tmoments)
+    return fail(-1, "null argument%s", "");
+  if (nt < 1) return fail(-1, "lsm tangents: nt must be positive%s", "");
+  if (d_imm && (!d_xi || !d_ni || !d_dni || !d_dimm)) return fail(-1, "lsm tangents: exercise update needs its arrays%s", "");
+  if (chunk_paths <= 0 || chunk_paths % 256 != 0) return fail(-2, "lsm: chunk_paths must be a positive multiple of 256%s", "");
+  cudaStream_t st = (cudaStream_t)stream;
+  const int nv = 4 + 5 * n_rights;
+  if (n <= 0) {
+    MCRE_CUDA(cudaMemsetAsync(d_tmoments, 0, (size_t)nt * nv * sizeof(double), st));
+    return 0;
+  }
+  const long long n_chunks = (n + chunk_paths - 1) / chunk_paths;
+  long long gx = (long long)sm_count() * 4;
+  if (gx > n_chunks) gx = n_chunks;
+  dim3 grid((unsigned)gx, (unsigned)nt);
+  LsmCoef cf;
+  for (int s = 0; s < LSM_MAX_RIGHTS; ++s)
+    for (int j = 0; j < 3; ++j) cf.c[s][j] = (coef_i && s < n_rights) ? coef_i[s * 3 + j] : 0.0;
+#define LSM_TAN_LAUNCH(RV)                                                                                              \
+  lsm_step_states_tan_kernel<RV><<<grid, 256, 0, st>>>(nt, d_xk, d_nk, d_dxk, d_dnk, shift_k, scale_k, d_xi, d_ni, d_imm, \
+                                                       d_dni, d_dimm, coef_i != nullptr, cf, shift_i, scale_i, d_value,  \
+                                                       d_dvalue, n, chunk_paths, d_partial)
+  if (n_rights == 2) LSM_TAN_LAUNCH(2); else if (n_rights == 3) LSM_TAN_LAUNCH(3); else if (n_rights == 4) LSM_TAN_LAUNCH(4);
+  else if (n_rights == 5) LSM_TAN_LAUNCH(5); else LSM_TAN_LAUNCH(6);
+#undef LSM_TAN_LAUNCH
+  MCRE_LAUNCHED();
+  return mcre_tree_reduce(d_partial, n_chunks, (int64_t)nt * nv, d_tmoments, stream);
 }
 
 extern "C" int mcre_lsm_step_states(int32_t n_rights, const double *d_xk, const double *d_nk, double shift_k,

@@ -73,9 +73,9 @@ SYMBOLS = [
     "mcre_irc_create", "mcre_irc_destroy", "mcre_irc_main_slots", "mcre_irc_presim_slots",
     "mcre_irc_presim_scratch_bytes", "mcre_irc_partial_bytes", "mcre_irc_presim", "mcre_irc_presim_tangent_slots",
     "mcre_irc_set_coefficients", "mcre_irc_solve_coefficients", "mcre_irc_set_coefficients_device", "mcre_irc_mainsim", "mcre_irc_set_pv_spill", "mcre_irc_set_path_replay", "mcre_select_locate",
-    "mcre_irc_set_exercise_coefficients", "mcre_irc_lsm_scratch_bytes", "mcre_irc_lsm_forward", "mcre_lsm_step", "mcre_lsm_step_states", "mcre_lsm_step_dev", "mcre_lsm_solve_dev", "mcre_lsm_moments_batch", "mcre_lsm_step_batch", "mcre_lsm_step_tangents",
-    "mcre_lsm_prepare_equity",
-    "mcre_eq_create", "mcre_eq_destroy", "mcre_eq_slots", "mcre_eq_mainsim", "mcre_eq_presim", "mcre_eq_presim_tangents", "mcre_eq_set_exposure_coef_tangents", "mcre_eq_set_credit", "mcre_eq_set_cva_weight_spill", "mcre_eq_cva_paths", "mcre_eq_set_pv_accumulator", "mcre_eq_set_bridge_uniforms", "mcre_eq_set_exposure_accumulator", "mcre_eq_set_exposure_tangent_accumulator", "mcre_exposure_tangent_sums", "mcre_exposure_tangent_sums_paths", "mcre_eq_credit_weight_tangents", "mcre_eq_unsecured_exposures", "mcre_sum_stats",
+    "mcre_irc_set_exercise_coefficients", "mcre_irc_lsm_scratch_bytes", "mcre_irc_lsm_forward", "mcre_lsm_step", "mcre_lsm_step_states", "mcre_lsm_step_dev", "mcre_lsm_solve_dev", "mcre_lsm_moments_batch", "mcre_lsm_step_batch", "mcre_lsm_step_tangents", "mcre_lsm_step_states_tangents",
+    "mcre_lsm_prepare_equity", "mcre_lsm_prepare_equity_tangents",
+    "mcre_eq_create", "mcre_eq_destroy", "mcre_eq_slots", "mcre_eq_mainsim", "mcre_eq_presim", "mcre_eq_presim_tangents", "mcre_eq_set_exposure_coef_tangents", "mcre_eq_set_exercise_exposure_coef_tangents", "mcre_eq_set_credit", "mcre_eq_set_cva_weight_spill", "mcre_eq_cva_paths", "mcre_eq_set_pv_accumulator", "mcre_eq_set_bridge_uniforms", "mcre_eq_set_exposure_accumulator", "mcre_eq_set_exposure_tangent_accumulator", "mcre_exposure_tangent_sums", "mcre_exposure_tangent_sums_paths", "mcre_eq_credit_weight_tangents", "mcre_eq_unsecured_exposures", "mcre_sum_stats",
     "mcre_storage_create", "mcre_storage_destroy", "mcre_storage_spots", "mcre_storage_backward", "mcre_storage_moment_slots", "mcre_storage_moments", "mcre_storage_solve", "mcre_storage_mainsim",
     "mcre_select_create", "mcre_select_destroy", "mcre_select_begin", "mcre_select_count",
     "mcre_select_scan", "mcre_select_compact", "mcre_select_finish",
@@ -137,6 +137,10 @@ def lib():
                                          C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, c_dp, C.c_double,
                                          C.c_double, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p,
                                          C.c_void_p]
+    L.mcre_lsm_step_states_tangents.argtypes = [C.c_int32] + list(L.mcre_lsm_step_tangents.argtypes)
+    L.mcre_lsm_prepare_equity_tangents.argtypes = [C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_int32, c_ip, c_dp,
+                                                   C.c_int32, C.c_int32, C.c_int32, c_ip, C.c_int32, C.c_double,
+                                                   C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     L.mcre_eq_create.argtypes = [C.c_void_p, C.POINTER(C.c_void_p)]
     L.mcre_eq_destroy.argtypes = [C.c_void_p]
     L.mcre_eq_destroy.restype = None
@@ -148,6 +152,7 @@ def lib():
                                  C.c_void_p, C.c_void_p]
     L.mcre_eq_presim_tangents.argtypes = [C.c_void_p, C.POINTER(Rng), C.POINTER(Shard)] + [C.c_void_p] * 7
     L.mcre_eq_set_exposure_coef_tangents.argtypes = [C.c_void_p, c_dp]
+    L.mcre_eq_set_exercise_exposure_coef_tangents.argtypes = [C.c_void_p, c_dp]
     L.mcre_eq_set_credit.argtypes = [C.c_void_p, C.c_void_p]
     L.mcre_eq_set_cva_weight_spill.argtypes = [C.c_void_p, C.c_void_p]
     L.mcre_eq_cva_paths.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_double, C.c_void_p, C.c_void_p]

@@ -226,6 +226,7 @@ class EquityBackend:
         self.id_to_asset = {a.asset_id: i for i, a in enumerate(self.assets)}
         self.exercise_coef = {}        # id(product) -> (coef [n_ex, rights, 3] standardised basis, basis [n_ex, 2])
         self.exercise_expo_coef = {}   # id(product) -> (coef [n_expo, rights, 3], basis [n_expo, 2]) per exposure date
+        self.exercise_expo_dcoef = {}  # id(product) -> d coef / d (lane parameters of the product's asset) [n_expo, rights, nt, 3]
         self.expo_coef = {}       # id(product) -> (coef [n_expo, 3] standardised basis, basis [n_expo, 2])
         self.expo_dcoef = {}      # id(product) -> d coef / d (lane parameters of the product's asset) [n_expo, nt, 3]
         subs = _sub_models(ctrl.model)
@@ -443,10 +444,11 @@ class EquityBackend:
             step_chol.append(seen[key])
         return 1, None, chol_dual, step_chol
 
-    def lower(self, set_indices, presim_products=None, subset=None, presim_tangents=False):
+    def lower(self, set_indices, presim_products=None, subset=None, presim_tangents=False, spill_times=None):
         """Plan of the main pass for a group of netting sets, or (presim_products given) of the
         pre-simulation spill pass for a group of products (all in one dummy set).  `subset`: the
-        products to keep (book splitting: one launch evaluates a part of a large netting set)."""
+        products to keep (book splitting: one launch evaluates a part of a large netting set).
+        `spill_times` (spill pass): the dates to spill spots at instead of the exposure dates."""
         c, nt, A = self.c, self.nt, self.A
         if presim_products is not None and not presim_tangents:
             nt = 0
@@ -590,15 +592,16 @@ class EquityBackend:
                     raise NotImplementedError("sensitivities of exposure profiles of equity books: one Black-Scholes "
                                               "model (single or multi-asset) or one Heston model")
                 for p in owners:
-                    if c._can_use_analytic_exposure_for_product(p):
-                        continue
-                    if is_equity_exercise(p) or id(p) not in self.expo_dcoef:
-                        raise NotImplementedError("sensitivities of exposure profiles of equity books: European "
-                                                  "options (analytic exposure) and single-asset products that pay once "
-                                                  "(regression proxy); not exercise products or baskets")
+                    if c._can_use_analytic_exposure_for_product(p) or is_equity_exercise(p):
+                        continue      # (exercise products: tangent backward induction, exercise_expo_dcoef)
+                    if id(p) not in self.expo_dcoef:
+                        raise NotImplementedError("sensitivities of exposure profiles of equity books: not implemented for "
+                                                  "baskets (regression proxies on several assets)")
                 if any(m.metric_type == MetricType.PFE for m in c.risk_metrics.metrics) and not getattr(c, "_credit_passenger", False):
                     raise NotImplementedError("PFE sensitivities are not implemented for equity books")
             expo_times, metric_times = c.exposure_timeline.tolist(), c.metric_exposure_timeline.tolist()
+            if spill_times is not None:
+                expo_times = list(spill_times)
             n_expo, n_metric = len(expo_times), len(metric_times)
             date_expo = np.full(n_dates, -1, dtype=np.int32)
             date_metric = np.full(n_dates, -1, dtype=np.int32)
@@ -608,6 +611,7 @@ class EquityBackend:
                 date_metric[date_idx[tm]] = m
             xp = np.zeros((n_expo, max(len(recs), 1), EQ_XP))
             xp_tan = np.zeros((n_expo, max(len(recs), 1), 3, max(nt, 1))) if (nt and presim_products is None) else None
+            xp_ex_tan = None      # [n_expo][n_prod][EQ_MAX_RIGHTS][3][nt], exercise products only
             # per product, all exposure dates at once (books of thousands of products x ~100 dates: no Python in the
             # (date, product) loop)
             te_arr = np.asarray(expo_times, dtype=np.float64)
@@ -629,6 +633,12 @@ class EquityBackend:
                     xp[on, pi, 5], xp[on, pi, 6] = basis[on, 0], basis[on, 1]
                     for st in range(1, coef.shape[1]):
                         xp[on, pi, 16 + 3 * (st - 1):19 + 3 * (st - 1)] = coef[on, st]
+                    xp[on, pi, 7] = dinv[on]
+                    if xp_tan is not None:
+                        if xp_ex_tan is None:
+                            xp_ex_tan = np.zeros((n_expo, len(recs), EQ_MAX_RIGHTS, 3, nt))
+                        dcoef = self.exercise_expo_dcoef[id(p)]                  # [n_expo, rights, nt, 3]
+                        xp_ex_tan[on, pi, :coef.shape[1]] = np.transpose(dcoef[on], (0, 1, 3, 2))
                 else:
                     coef, basis = self.expo_coef[id(p)]              # [n_expo, 3], [n_expo, 2]
                     on = np.any(coef != 0.0, axis=1)
@@ -666,7 +676,8 @@ class EquityBackend:
             desc.set_flags, desc.set_lag = ip("set_flags", set_flags), ip("set_lag", set_lag)
         desc.n_expo, desc.n_metric, desc.acc_flags = n_expo, n_metric, acc
         info = dict(grid=grid, noise_dim=d, n_uniform=desc.n_uniform, owners=owners, recs=recs, n_metric=n_metric, acc=acc,
-                    bridge=bridge, chol=chol, set_indices=list(set_indices), xp_tan=xp_tan if (n_expo and presim_products is None) else None)
+                    bridge=bridge, chol=chol, set_indices=list(set_indices), xp_tan=xp_tan if (n_expo and presim_products is None) else None,
+                    xp_ex_tan=xp_ex_tan if (n_expo and presim_products is None) else None)
         return desc, t, info
 
     def _set_credit(self, plan, info):
@@ -821,21 +832,35 @@ class EquityBackend:
             return
         c = self.c
         n_expo = len(c.exposure_timeline) if c.risk_metrics.requires_exposure_profiles() else 0
+        nt = self.nt if n_expo else 0       # tangents of the induction: sensitivities of exposure metrics only
         _, count = RT.shard_range(c.num_paths_presim, CHUNK_PATHS)
-        per_product = max((3 * (len(p.product_timeline) + n_expo) + 2) * max(count, 1) * 8 for p in prods)
+        # value arrays (xs, nums, imm) + f32 values; with tangents dxs, dnums, dimm, the running tangents and the
+        # product's share of the tangent spill of every asset
+        per_product = max(((3 + nt * (3 + self.A)) * (len(p.product_timeline) + n_expo) + 2 + 2 * nt * p.num_exercise_rights)
+                          * max(count, 1) * 8 for p in prods)
         batch = max(1, min(64, int(6e9 // per_product)))
+        expo_times = c.exposure_timeline.tolist() if n_expo else []
         for b0 in range(0, len(prods), batch):
             group = prods[b0:b0 + batch]
-            prepared = [self.presim_exercise(p, dev, prepare_only=True) for p in group]
+            spill = None
+            if nt:
+                times = {t for p in group for t in p.regression_timeline.tolist() + p.product_timeline.tolist()}
+                spill = self.presim_tangent_spill(times | set(expo_times), dev)
+            prepared = [self.presim_exercise(p, dev, prepare_only=True, spill=spill) for p in group]
             coefs = run_backward_inductions([g for g, _ in prepared])
             for (_, finish), coef in zip(prepared, coefs):
                 finish(coef)
+            del spill, prepared
         self._presim_paths = None
 
-    def presim_exercise(self, prod, dev, prepare_only=False):
+    def presim_exercise(self, prod, dev, prepare_only=False, spill=None):
         """Longstaff-Schwartz pre-simulation of a Bermudan / American / FlexiCall option on equity underlyings
         (controller.py:294-383): pre-simulation paths from the path generator (seed 42), gathered
         date-major by mcre_lsm_prepare_equity, then the shared backward induction (mcre/lsm.py).
+        With tangents and exposure metrics the induction also differentiates the exposure coefficients: the tangents
+        of the gathered arrays come from the tangent spill of the pre-simulation (`spill` = presim_tangent_spill of
+        dates covering the product's regression dates, else one of its own) through mcre_lsm_prepare_equity_tangents;
+        the value arrays, and so every exercise decision and coefficient, are those of the value-only run.
         prepare_only: return (generator of the backward induction, finish(coef)) for the lock-step driver."""
         from mcre import paths as P
         from mcre.lsm import backward_induction_steps, run_backward_inductions, to_raw_basis
@@ -891,12 +916,32 @@ class EquityBackend:
             cols[xi][0], cols[xi][1], 1, ip([cols[ui][0]]), fp([1.0]), ip([cols[ui][1]]), 0.0, fp(exercise_strikes(prod)), sign,
             xs.data_ptr(), nums.data_ptr(), imm.data_ptr(), RT.stream_ptr()))
         del paths
+        tangents = None
+        nt = self.nt if expo_times else 0
+        if nt:
+            if xi != ui:
+                raise NotImplementedError("sensitivities of exposure profiles of exercise products: the explanatory "
+                                          "variable must be the underlying's spot")
+            dx, rows = spill if spill is not None else self.presim_tangent_spill(reg_times, dev)
+            tbuf = torch.empty((2 * n_reg + n_ex) * nt * n, dtype=torch.float64, device=dev)
+            dxs = tbuf[:n_reg * nt * n].view(n_reg, nt, n)
+            dnums = tbuf[n_reg * nt * n:2 * n_reg * nt * n].view(n_reg, nt, n)
+            dimm = tbuf[2 * n_reg * nt * n:].view(n_ex, nt, n)
+            # d numeraire / d rate = (t - t0) exp(r (t - t0)), on the lane's rate (parameter 2, the numeraire's rate)
+            B.check(L.mcre_lsm_prepare_equity_tangents(
+                dx.data_ptr(), count, self.A, nt, n_reg, ip([rows[t] for t in reg_times]),
+                fp([(t - t0) * math.exp(self.num_rate * (t - t0)) for t in reg_times]), 2, xi, n_ex,
+                ip([rows[t] for t in ptl]), ui, sign, imm.data_ptr(), dxs.data_ptr(), dnums.data_ptr(), dimm.data_ptr(),
+                RT.stream_ptr()))
+            del dx
+            tangents = dict(nt=nt, dxs=dxs, dnums=dnums, dimm=dimm)
         # standardisation of the explanatory variable per date: model moments (shard independent)
         basis = np.array([self.basis_at(xi, t) for t in reg_times]).reshape(n_reg, 2)
         gen = backward_induction_steps(xs, nums, imm, ptl, reg_times, basis, count, CHUNK_PATHS, dev, n_rights=R,
-                                       batched=prepare_only)
+                                       tangents=tangents, batched=prepare_only)
 
-        def finish(coef):
+        def finish(out):
+            coef, dcoef = out if tangents is not None else (out, None)
             coef = coef.reshape(n_reg, R, 3)
             ridx = {t: k for k, t in enumerate(reg_times)}
             rows = [ridx[t] for t in ptl]
@@ -911,10 +956,59 @@ class EquityBackend:
                 erows = [ridx[t] for t in expo_times]
                 self.exercise_expo_coef[id(prod)] = (coef[erows], basis[erows])
                 c.regression_coeffs[prod.product_id][:, 1:R + 1, :] = torch.tensor(raw[erows])
+                if dcoef is not None:
+                    self.exercise_expo_dcoef[id(prod)] = dcoef.reshape(n_reg, R, nt, 3)[erows]
 
         if prepare_only:
             return gen, finish
         finish(run_backward_inductions([gen])[0])
+
+    def _presim_rng(self, dev):
+        """Draws of the pre-simulation (seed 42): Philox, or the injected reference stream."""
+        c = self.c
+        inj = c.injected_normals.get("pre") if c.injected_normals else None
+        rng = B.Rng()
+        rng.seed, rng.stream, rng.n_paths_total = 42, c.rng_stream, c.num_paths_presim
+        if inj is not None:
+            rng.mode, rng.d_z = B.RNG_INJECT, inj.data_ptr()
+            iu = getattr(c, "injected_uniforms", None)
+            iu = iu.get("pre") if iu else None
+            if iu is not None:
+                self._keep_u_pre = torch.as_tensor(iu, dtype=torch.float64).to(dev).contiguous()
+                rng.d_u = self._keep_u_pre.data_ptr()
+        else:
+            rng.mode = B.RNG_PHILOX
+        return rng
+
+    def presim_tangent_spill(self, times, dev):
+        """Pathwise tangents of every asset's spot at `times` on the pre-simulation paths: the spill pass of the fused
+        kernel (mcre_eq_presim_tangents) on a plan without products whose spill dates are `times`, replaying the
+        pre-simulation draws with tangents (under EULER the sub-steps between dates are not stored, so the tangents
+        cannot come from the materialised paths).  -> (dx [len(times), A, nt, n] device, {time: row})."""
+        c, L = self.c, B.lib()
+        n_pre = c.num_paths_presim
+        begin, count = RT.shard_range(n_pre, CHUNK_PATHS)
+        n = max(count, 1)
+        times = sorted(set(times))
+        x = torch.zeros((len(times), self.A, n), dtype=torch.float64, device=dev)
+        dx = torch.zeros((len(times), self.A, self.nt, n), dtype=torch.float64, device=dev)
+        cf = torch.zeros(1, dtype=torch.float32, device=dev)          # (no products: no cashflows)
+        dcf = torch.zeros(1, dtype=torch.float64, device=dev)
+        desc, keep, info = self.lower([], presim_products=[], presim_tangents=True, spill_times=times)
+        plan = C.c_void_p()
+        B.check(L.mcre_eq_create(C.byref(desc), C.byref(plan)))
+        try:
+            slots = L.mcre_eq_slots(plan)
+            spill_chunk = main_chunk(n_pre)
+            partial = torch.empty(((n + spill_chunk - 1) // spill_chunk) * slots + slots + 1, dtype=torch.float64, device=dev)
+            shift = torch.zeros(slots, dtype=torch.float64, device=dev)
+            rng = self._presim_rng(dev)
+            sh = B.Shard(begin, count, spill_chunk)
+            B.check(L.mcre_eq_presim_tangents(plan, C.byref(rng), C.byref(sh), partial.data_ptr(), shift.data_ptr(),
+                                              x.data_ptr(), cf.data_ptr(), dx.data_ptr(), dcf.data_ptr(), RT.stream_ptr()))
+        finally:
+            L.mcre_eq_destroy(plan)
+        return dx, {t: i for i, t in enumerate(times)}
 
     def presim_regression(self, products, dev):
         """Regression-proxy exposure coefficients of products that pay once (controller.py:294-383): the
@@ -956,7 +1050,6 @@ class EquityBackend:
             trk += t
         if cur:
             groups.append(cur)
-        inj = c.injected_normals.get("pre") if c.injected_normals else None
         for group in groups:
             desc, keep, info = self.lower([], presim_products=group, presim_tangents=bool(nt))
             plan = C.c_void_p()
@@ -970,17 +1063,7 @@ class EquityBackend:
                 spill_chunk = main_chunk(n_pre)
                 partial = torch.empty(((n + spill_chunk - 1) // spill_chunk) * slots + slots + 1, dtype=torch.float64, device=dev)
                 shift = torch.zeros(slots, dtype=torch.float64, device=dev)
-                rng = B.Rng()
-                rng.seed, rng.stream, rng.n_paths_total = 42, c.rng_stream, n_pre
-                if inj is not None:
-                    rng.mode, rng.d_z = B.RNG_INJECT, inj.data_ptr()
-                    iu = getattr(c, "injected_uniforms", None)
-                    iu = iu.get("pre") if iu else None
-                    if iu is not None:
-                        self._keep_u_pre = torch.as_tensor(iu, dtype=torch.float64).to(dev).contiguous()
-                        rng.d_u = self._keep_u_pre.data_ptr()
-                else:
-                    rng.mode = B.RNG_PHILOX
+                rng = self._presim_rng(dev)
                 keep_bridge = self._set_bridge_uniforms(plan, info, "pre", n_pre, dev)
                 sh = B.Shard(begin, count, spill_chunk)
                 if nt:
@@ -1062,6 +1145,17 @@ class EquityBackend:
         for p in products:
             coef, basis = self.expo_coef[id(p)]
             c.regression_coeffs[p.product_id][:, 0, :] = torch.tensor(to_raw_basis(coef, basis, [t <= t0 for t in expo_times]))
+
+    @staticmethod
+    def _set_coef_tangents(plan, info):
+        """Hands a plan with tangents the coefficient tangents of its regression-proxy and exercise exposures."""
+        L = B.lib()
+        if info.get("xp_tan") is not None:
+            _, ptr = B.as_dp(info["xp_tan"].reshape(-1))     # (copied to the device by the call)
+            B.check(L.mcre_eq_set_exposure_coef_tangents(plan, ptr))
+        if info.get("xp_ex_tan") is not None:
+            _, ptr = B.as_dp(info["xp_ex_tan"].reshape(-1))
+            B.check(L.mcre_eq_set_exercise_exposure_coef_tangents(plan, ptr))
 
     def _set_bridge_uniforms(self, plan, info, which, n_total, dev):
         """RNG compatibility mode: hand the launch the reference's numpy uniforms of its Brownian-bridge barrier
@@ -1260,9 +1354,7 @@ class EquityBackend:
                 B.check(L.mcre_eq_set_pv_accumulator(plan, accum.data_ptr()))
                 B.check(L.mcre_eq_set_exposure_accumulator(plan, accum_e.data_ptr()))
                 B.check(L.mcre_eq_set_exposure_tangent_accumulator(plan, accum_t.data_ptr()))
-                if info.get("xp_tan") is not None:
-                    keep_xt, xt_ptr = B.as_dp(info["xp_tan"].reshape(-1))
-                    B.check(L.mcre_eq_set_exposure_coef_tangents(plan, xt_ptr))
+                self._set_coef_tangents(plan, info)
                 keep_bridge = self._set_bridge_uniforms(plan, info, "main", n_main, dev)
                 rng = self._rng(43, n_main)
                 sh = B.Shard(begin, count, chunk)
@@ -1334,9 +1426,8 @@ class EquityBackend:
                 partial = torch.empty(n_chunks * slots + 1, dtype=torch.float64, device=dev)
                 rng = self._rng(43, n_main)
                 keep_bridge = self._set_bridge_uniforms(plan, info, "main", n_main, dev)
-                if info.get("xp_tan") is not None and self.nt:
-                    keep_xt, xt_ptr = B.as_dp(info["xp_tan"].reshape(-1))
-                    B.check(L.mcre_eq_set_exposure_coef_tangents(plan, xt_ptr))
+                if self.nt:
+                    self._set_coef_tangents(plan, info)
                 sh = B.Shard(begin, count, chunk)
                 n_metric = info["n_metric"]
                 spill = None

@@ -113,6 +113,12 @@ def regression_tangents(G, rhs, coef, tm):
     return out
 
 
+def state_tangent_moments(tm, s):
+    """Tangent moments of state s (0-based: s + 1 rights left) in the layout regression_tangents takes, [nt, 9], from
+    the multi-state layout of mcre_lsm_step_states_tangents [nt, 4 + 5 R] (sum u^m du shared by the states)."""
+    return np.concatenate([tm[:, :4], tm[:, 4 + 5 * s:9 + 5 * s]], axis=1)
+
+
 LSM_MAX_RIGHTS = 6         # MCRE_LSM_MAX_RIGHTS (include/mcre.h)
 LSM_MAX_NV = 5 + 3 * LSM_MAX_RIGHTS   # moments of the widest step
 
@@ -144,9 +150,12 @@ def backward_induction_steps(xs, nums, imm, ptl, reg_times, basis, count, chunk_
     dates; reg_times: regression dates (sorted, contain every product date); basis: [n_reg, 2] (shift, scale).
     -> coefficients in the standardised basis: [n_reg, 3] for one exercise right, [n_reg, n_rights, 3]
     (state s = rights left at row s-1) for a FlexiCall.
-    tangents (one exercise right): dict(nt, dxs [n_reg, nt, n], dnums [n_reg, nt, n], dimm [n_ex, nt, n]) - the
-    pathwise tangents of the spilled arrays; the generator then also returns d(coefficients)/d(parameters)
-    [n_reg, nt, 3] (mcre_lsm_step_tangents + regression_tangents): -> (coef, dcoef)."""
+    tangents: dict(nt, dxs [n_reg, nt, n], dnums [n_reg, nt, n], dimm [n_ex, nt, n]) - the pathwise tangents of the
+    spilled arrays; the generator then also returns d(coefficients)/d(parameters) (mcre_lsm_step_states_tangents +
+    regression_tangents once per state, with the state's right-hand side, coefficients and tangent moments):
+    -> (coef, dcoef), dcoef [n_reg, nt, 3] for one exercise right, [n_reg, n_rights, nt, 3] otherwise.  Tangent
+    products step through the per-product launches (the exercise decisions, and so the coefficients, are those of the
+    batched launch bit for bit)."""
     L = B.lib()
     stream = RT.stream_ptr()      # once per induction: tens of thousands of steps per book
     n_reg = len(reg_times)
@@ -161,13 +170,13 @@ def backward_induction_steps(xs, nums, imm, ptl, reg_times, basis, count, chunk_
     moments = torch.zeros(LSM_MAX_NV, dtype=torch.float64, device=dev)
     keep = {}
     if tangents is not None:
-        assert R == 1, "tangents of the regression: one exercise right"
         nt = int(tangents["nt"])
+        ntv = 4 + 5 * R       # tangent moments per parameter: sum u^m du, then 5 per state
         dxs, dnums, dimm = tangents["dxs"], tangents["dnums"], tangents["dimm"]
-        dvalue = torch.zeros((nt, n), dtype=torch.float64, device=dev)
-        tpartial = torch.empty(n_chunks * nt * 9 + 1, dtype=torch.float64, device=dev)
-        tmoments = torch.zeros(nt * 9, dtype=torch.float64, device=dev)
-        dcoef = np.zeros((n_reg, nt, 3))
+        dvalue = torch.zeros((R, nt, n), dtype=torch.float64, device=dev)
+        tpartial = torch.empty(n_chunks * nt * ntv + 1, dtype=torch.float64, device=dev)
+        tmoments = torch.zeros(nt * ntv, dtype=torch.float64, device=dev)
+        dcoef = np.zeros((n_reg, R, nt, 3))
 
     batched = batched and tangents is None
     queue = []
@@ -206,10 +215,10 @@ def backward_induction_steps(xs, nums, imm, ptl, reg_times, basis, count, chunk_
             if i is not None:
                 targs = (args_i[0], args_i[1], args_i[2], dnums[ki].data_ptr(), dimm[i].data_ptr(), args_i[3],
                          args_i[4], args_i[5])
-            B.check(L.mcre_lsm_step_tangents(nt, xs[k].data_ptr(), nums[k].data_ptr(), dxs[k].data_ptr(),
-                                             dnums[k].data_ptr(), float(basis[k, 0]), float(basis[k, 1]), *targs,
-                                             value.data_ptr(), dvalue.data_ptr(), count, chunk_paths,
-                                             tpartial.data_ptr(), tmoments.data_ptr(), stream))
+            B.check(L.mcre_lsm_step_states_tangents(R, nt, xs[k].data_ptr(), nums[k].data_ptr(), dxs[k].data_ptr(),
+                                                    dnums[k].data_ptr(), float(basis[k, 0]), float(basis[k, 1]), *targs,
+                                                    value.data_ptr(), dvalue.data_ptr(), count, chunk_paths,
+                                                    tpartial.data_ptr(), tmoments.data_ptr(), stream))
 
     last = len(ptl)
     for k in range(n_reg - 1, -1, -1):
@@ -233,11 +242,12 @@ def backward_induction_steps(xs, nums, imm, ptl, reg_times, basis, count, chunk_
             solved, m = yield moments   # [3 states, 3] from the driver's batched solve of this round, host moments
         coef[k] = solved[:R]
         if tangents is not None:
-            tm = RT.all_reduce_tree(tmoments).cpu().numpy().reshape(nt, 9)
+            tm = RT.all_reduce_tree(tmoments).cpu().numpy().reshape(nt, ntv)
             G = np.array([[m[0], m[1], m[2]], [m[1], m[2], m[3]], [m[2], m[3], m[4]]])
-            dcoef[k] = regression_tangents(G, m[5:8], coef[k, 0], tm)
+            for s in range(R):
+                dcoef[k, s] = regression_tangents(G, m[5 + 3 * s:8 + 3 * s], coef[k, s], state_tangent_moments(tm, s))
     if tangents is not None:
-        return coef[:, 0, :], dcoef
+        return (coef[:, 0, :], dcoef[:, 0]) if R == 1 else (coef, dcoef)
     return coef[:, 0, :] if R == 1 else coef
 
 
