@@ -356,9 +356,9 @@ __global__ void __launch_bounds__(32) storage_solve_kernel(int S, int NB, const 
     for (int a = 0; a < NB; ++a)
       for (int b = 0; b < NB; ++b) { G[a][b] = mom[S * NB + a + b]; V[a][b] = a == b ? 1.0 : 0.0; }
     for (int a = 0; a < NB; ++a) dmax = fmax(dmax, G[a][a]);
-    // fast path: a Cholesky factorisation whose pivots stay above 1e-8 of the largest diagonal entry - the matrix is
-    // then far from the rcond cut-off and the pseudo-inverse is the inverse (all but the deterministic-spot dates;
-    // the single-thread Jacobi sweeps below cost 80 us, as much as the backward and moments kernels together)
+    // fast path: a Cholesky factorisation whose pivots stay above 1e-8 of the largest diagonal entry and whose inverse
+    // certifies that no eigenvalue is cut: the pseudo-inverse is then the inverse (all but the deterministic-spot
+    // dates; the single-thread Jacobi sweeps below cost 80 us, as much as the backward and moments kernels together)
     int ok = 1;
     for (int j = 0; j < NB && ok; ++j) {
       double d = G[j][j];
@@ -371,6 +371,31 @@ __global__ void __launch_bounds__(32) storage_solve_kernel(int S, int NB, const 
         for (int k = 0; k < j; ++k) v -= Lc[i][k] * Lc[j][k];
         Lc[i][j] = v / lj;
       }
+    }
+    // The pivots bound the smallest eigenvalue from above only: Hankel moments of a few support points pass them with
+    // lambda_min / lambda_max far below rcond.  So the fast path also needs the lower bound lambda_min >= 1 / |G^-1|_F
+    // (G^-1 = L^-T L^-1 from the factor) to exceed rcond * trace(G) >= rcond * lambda_max; otherwise the Jacobi path
+    // below applies the cut-off.
+    if (ok) {
+      double Li[ST_MAX_B][ST_MAX_B];       // L^-1 (lower triangular)
+      for (int j = 0; j < NB; ++j) {
+        Li[j][j] = 1.0 / Lc[j][j];
+        for (int i = j + 1; i < NB; ++i) {
+          double v = 0.0;
+          for (int k = j; k < i; ++k) v += Lc[i][k] * Li[k][j];
+          Li[i][j] = -v / Lc[i][i];
+        }
+      }
+      double fro = 0.0, trace = 0.0;
+      for (int a = 0; a < NB; ++a) {
+        trace += G[a][a];
+        for (int b = 0; b < NB; ++b) {
+          double v = 0.0;
+          for (int k = a > b ? a : b; k < NB; ++k) v += Li[k][a] * Li[k][b];
+          fro += v * v;
+        }
+      }
+      ok = 1.0 / sqrt(fro) > rcond * trace;
     }
     use_chol = ok;
     for (int sweep = 0; sweep < 12 && !ok; ++sweep) {

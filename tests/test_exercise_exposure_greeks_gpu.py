@@ -178,10 +178,16 @@ def _tangent_step(L, R, nt, d, coef, value, dvalue, chunk, entry="states"):
 def test_multi_right_tangent_step_matches_numpy(R):
     """mcre_lsm_step_states_tangents on random inputs after the value step of the same date: the running tangents and
     the tangent moments against a numpy restatement of the update (decisions from the value step's expressions) and of
-    the sums at 1e-12; one right is mcre_lsm_step_tangents bit for bit."""
+    the sums at 1e-12; one right is mcre_lsm_step_tangents bit for bit.  9000 paths in 4096-path chunks, and more
+    256-path chunks than the kernel's grid cap of sm_count * 4 blocks, so that blocks loop over several chunks."""
+    sm = torch.cuda.get_device_properties(0).multi_processor_count
+    for n, chunk in ((9000, 4096), ((4 * sm + 3) * 256 + 17, 256)):
+        _check_tangent_step(R, 3, n, chunk)
+
+
+def _check_tangent_step(R, nt, n, chunk):
     from mcre import binding as B
     L = B.lib()
-    nt, n, chunk = 3, 9000, 4096
     d, coef = _step_inputs(R, nt, n, 11 + R)
     value = d["value"].clone()
     n_chunks = (n + chunk - 1) // chunk
