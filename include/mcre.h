@@ -226,7 +226,11 @@ int64_t mcre_irc_partial_bytes(const mcre_irc_plan *plan, int64_t n_paths, int32
  * x, N and the windowed cashflows and d_tmoments receives [n_units][nt][n_reg][9] =
  * sum u^m du (m = 0..3), sum u^i dY (i = 0..2), sum du Y, sum 2 u du Y, from which the host
  * differentiates the normal equations.  d_tmoments may be NULL for nt = 0.
- * d_scratch / d_partial sized by the helpers above. */
+ * d_scratch / d_partial sized by the helpers above.
+ * A shard without paths (a rank that holds none of the pre-simulation's chunks) writes zeros to its
+ * mcre_irc_presim_slots moments and, with tangents, its mcre_irc_presim_tangent_slots tangent moments, so
+ * that callers need not pre-zero them before the all-reduce.  A plan whose regression dates do not fit the
+ * moment kernels' shared memory returns -3 before any kernel is launched. */
 int64_t mcre_irc_presim_tangent_slots(const mcre_irc_plan *plan);
 int mcre_irc_presim(mcre_irc_plan *plan, const mcre_rng *rng, const mcre_shard *shard,
                     void *d_scratch, double *d_partial, double *d_moments, double *d_tmoments, void *stream);

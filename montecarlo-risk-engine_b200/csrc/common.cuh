@@ -97,5 +97,6 @@ struct DevArray {
 };
 
 int sm_count();
+int smem_optin_limit();   // cudaDevAttrMaxSharedMemoryPerBlockOptin of the current device (cached)
 
 }  // namespace mcre

@@ -1102,7 +1102,7 @@ static int eq_launch(mcre_eq_plan *p, const RngDev &rng, const ShardDev &sh, dou
   if (n_chunks == 0 && presim) return 0;
   auto k = eq_main_kernel<KIND, ALT, NT, NS, XH>;
   // (14 KB of static function tables: static + dynamic shared memory beyond 48 KB needs the opt-in, before the query)
-  if (smem > 32 * 1024) MCRE_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  MCRE_SMEM(k, smem, "eq main kernel does not fit (%s%lld bytes of shared memory)");
   int per_sm = 1;
   MCRE_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, threads, smem));
   if (per_sm < 1) return fail(-3, "eq main kernel does not fit%s", "");
@@ -1111,7 +1111,6 @@ static int eq_launch(mcre_eq_plan *p, const RngDev &rng, const ShardDev &sh, dou
   // The pilot launch (global path 0 -> the common shift of the shifted sums) runs on every rank, also on one whose
   // shard is empty (fewer chunks than ranks): all ranks finish the all-reduced sums with the same shift.
   ShardDev pilot_sh{0, 1, sh.chunk};
-  if (smem > 32 * 1024) MCRE_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   if (!presim) {   // the pre-simulation pass only spills; it needs no pilot shifts
     k<<<1, threads, smem, st>>>(d, rng, pilot_sh, partial, shift, spill, 1);
     MCRE_LAUNCHED();

@@ -539,10 +539,7 @@ extern "C" int mcre_irc_set_coefficients(mcre_irc_plan *p, const double *coef, v
       // the CVA-only kernel mode evaluates the polynomial in the raw basis [1, r, r^2]:
       // c(u) with u = (r - shift) * scale  ->  c'(r)
       const double sh = p->h_date_rec[(size_t)di * DR + 4], sc = p->h_date_rec[(size_t)di * DR + 5];
-      const double c0 = r[0], c1 = r[1], c2 = r[2];
-      r[2] = c2 * sc * sc;
-      r[1] = c1 * sc - 2.0 * c2 * sc * sc * sh;
-      r[0] = c0 - c1 * sc * sh + c2 * sc * sc * sh * sh;
+      irc_raw_basis(r[0], r[1], r[2], sh, sc, r);
     }
   }
   MCRE_CUDA(cudaMemcpyAsync((void *)p->d.date_rec, p->h_date_rec.data(), p->h_date_rec.size() * sizeof(double),
@@ -661,8 +658,25 @@ extern "C" int mcre_irc_mainsim(mcre_irc_plan *p, const mcre_rng *rng, const mcr
 }
 
 // defined in irc_tan.cu
+int irc_presim_tangent_fit(const mcre_irc_plan *p);
 int irc_presim_tangent_pass(mcre_irc_plan *p, const mcre::RngDev &r, const mcre::ShardDev &sh, void *d_scratch,
                             double *d_partial, double *d_tmoments, cudaStream_t st);
+
+template <int NU>
+static int irc_presim_moments_launch(const IrcDev &d, const ShardDev &sh, size_t smem, const double *xbuf,
+                                     const double *nbuf, const float *wbuf, double *d_partial, cudaStream_t st) {
+  const int threads = 256;
+  auto k = irc_presim_moments_kernel<NU>;
+  int per_sm = 1;
+  MCRE_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, threads, smem));
+  if (per_sm < 1) return fail(-3, "irc presim kernel does not fit: too many regression dates%s", "");
+  const long long n_chunks = (sh.n_paths + sh.chunk - 1) / sh.chunk;
+  long long grid = (long long)sm_count() * per_sm;
+  if (grid > n_chunks) grid = n_chunks;
+  k<<<(unsigned)grid, threads, smem, st>>>(d, sh, xbuf, nbuf, wbuf, d_partial);
+  MCRE_LAUNCHED();
+  return 0;
+}
 
 extern "C" int mcre_irc_presim(mcre_irc_plan *p, const mcre_rng *rng, const mcre_shard *shard, void *d_scratch,
                                double *d_partial, double *d_moments, double *d_tmoments, void *stream) {
@@ -672,16 +686,35 @@ extern "C" int mcre_irc_presim(mcre_irc_plan *p, const mcre_rng *rng, const mcre
   if (p->d.nt != 0 && !d_tmoments) return fail(-1, "irc presim: the plan carries tangents but d_tmoments is null%s", "");
   if (rng->mode == MCRE_RNG_INJECT && !rng->d_z) return fail(-1, "inject mode without normals%s", "");
   const IrcDev &d = p->d;
-  if (d.n_reg == 0 || shard->n_paths == 0) return 0;
+  if (d.n_reg == 0) return 0;
+  cudaStream_t st = (cudaStream_t)stream;
+  // the moment kernels keep every regression date's sums in shared memory: a plan with too many dates is refused here,
+  // before anything is launched
+  const int nu = nu_template(d.n_units);
+  const int nv = 5 + 3 * nu, nw = 256 / 32;
+  const size_t smem = ((size_t)d.n_reg * nv + 2 * nw * nv) * sizeof(double);
+  const char *too_many = "irc presim kernel does not fit: too many regression dates (%s%lld bytes of shared memory)";
+  if (nu == 1) MCRE_SMEM(irc_presim_moments_kernel<1>, smem, too_many);
+  else if (nu == 2) MCRE_SMEM(irc_presim_moments_kernel<2>, smem, too_many);
+  else MCRE_SMEM(irc_presim_moments_kernel<4>, smem, too_many);
+  const bool tangents = d.nt != 0 && d.n_units > 0;
+  if (tangents) {
+    rc = irc_presim_tangent_fit(p);
+    if (rc) return rc;
+  }
+  if (shard->n_paths == 0) {
+    // a rank without pre-simulation paths contributes zero moments
+    MCRE_CUDA(cudaMemsetAsync(d_moments, 0, (size_t)mcre_irc_presim_slots(p) * sizeof(double), st));
+    if (tangents) MCRE_CUDA(cudaMemsetAsync(d_tmoments, 0, (size_t)mcre_irc_presim_tangent_slots(p) * sizeof(double), st));
+    return 0;
+  }
   RngDev r = make_rng(rng);
   ShardDev sh{shard->path_begin, shard->n_paths, shard->chunk_paths};
-  cudaStream_t st = (cudaStream_t)stream;
   const long long n = sh.n_paths;
   double *xbuf = (double *)d_scratch;
   double *nbuf = xbuf + (size_t)d.n_reg * n;
   float *wbuf = (float *)(nbuf + (size_t)d.n_reg * n);
-  const int threads = 256;
-  if (d.nt != 0 && d.n_units > 0) {
+  if (tangents) {
     // forward pass with tangents (fills the value buffers too) + tangent moments
     rc = irc_presim_tangent_pass(p, r, sh, d_scratch, d_partial, d_tmoments, st);
     if (rc) return rc;
@@ -699,23 +732,10 @@ extern "C" int mcre_irc_presim(mcre_irc_plan *p, const mcre_rng *rng, const mcre
 #undef LAUNCHF
     MCRE_LAUNCHED();
   }
-  const int nu = nu_template(d.n_units);
-  const int nv = 5 + 3 * nu, nw = threads / 32;
-  const size_t smem = ((size_t)d.n_reg * nv + 2 * nw * nv) * sizeof(double);
+  rc = nu == 1 ? irc_presim_moments_launch<1>(d, sh, smem, xbuf, nbuf, wbuf, d_partial, st)
+     : nu == 2 ? irc_presim_moments_launch<2>(d, sh, smem, xbuf, nbuf, wbuf, d_partial, st)
+               : irc_presim_moments_launch<4>(d, sh, smem, xbuf, nbuf, wbuf, d_partial, st);
+  if (rc) return rc;
   const long long n_chunks = (n + sh.chunk - 1) / sh.chunk;
-#define LAUNCHB(NUV)                                                                                     \
-  do {                                                                                                   \
-    auto k = irc_presim_moments_kernel<NUV>;                                                             \
-    if (smem > 32 * 1024) MCRE_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-    int per_sm = 1;                                                                                      \
-    MCRE_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, threads, smem));                 \
-    if (per_sm < 1) return fail(-3, "irc presim kernel does not fit: too many regression dates%s", "");  \
-    long long grid = (long long)sm_count() * per_sm;                                                     \
-    if (grid > n_chunks) grid = n_chunks;                                                                \
-    k<<<(unsigned)grid, threads, smem, st>>>(d, sh, xbuf, nbuf, wbuf, d_partial);                        \
-    MCRE_LAUNCHED();                                                                                     \
-  } while (0)
-  if (nu == 1) LAUNCHB(1); else if (nu == 2) LAUNCHB(2); else LAUNCHB(4);
-#undef LAUNCHB
   return mcre_tree_reduce(d_partial, n_chunks, mcre_irc_presim_slots(p), d_moments, stream);
 }

@@ -527,6 +527,23 @@ using namespace mcre;
 
 // Host copies of what the CVA-only kernel's event records are built from (irc_cva.cu)
 constexpr int CVA_REC = 24;        // doubles per event record
+
+// The CVA-only kernel evaluates the exposure polynomial in the raw basis [1, r, r^2]: c(u) with u = (r - shift) scale
+// becomes c'(r).  Every product and sum is rounded on its own (no FMA contraction on either side), so that the host
+// patch (mcre_irc_set_coefficients) and the device patch (irc_patch_coefficients_kernel) give the same bits.
+#ifdef __CUDA_ARCH__
+__device__ __forceinline__ double rn_mul(double a, double b) { return __dmul_rn(a, b); }
+__device__ __forceinline__ double rn_add(double a, double b) { return __dadd_rn(a, b); }
+#else
+inline double rn_mul(double a, double b) { volatile double r = a * b; return r; }
+inline double rn_add(double a, double b) { volatile double r = a + b; return r; }
+#endif
+__host__ __device__ inline void irc_raw_basis(double c0, double c1, double c2, double sh, double sc, double out[3]) {
+  const double c2s2 = rn_mul(rn_mul(c2, sc), sc), c1s = rn_mul(c1, sc);
+  out[2] = c2s2;
+  out[1] = rn_add(c1s, -rn_mul(rn_mul(2.0, c2s2), sh));
+  out[0] = rn_add(rn_add(c0, -rn_mul(c1s, sh)), rn_mul(rn_mul(c2s2, sh), sh));
+}
 struct CvaHost {
   int n_sub = 0, n_pre_dates = 0, n_metric = 0, vas_noise = 0, cir_noise = 1;
   double vas[4] = {0, 0, 0, 0}, cir[3] = {0, 0, 0}, chol[4] = {1, 0, 0, 1}, y0 = 0.0, lgd = 0.0;
@@ -577,7 +594,7 @@ static int launch_main(mcre_irc_plan *p, const RngDev &rng, const ShardDev &sh, 
   do {                                                                                                 \
     auto k = irc_main_kernel<NT, NS, CIRV, SCH, irc_pp(NT, NS), BERM>;                                 \
     /* (static shared memory: 14 KB of function tables; static + dynamic beyond 48 KB needs the opt-in) */ \
-    if (smem > 32 * 1024) MCRE_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+    MCRE_SMEM(k, smem, "irc main kernel does not fit: too many metric dates x tangents (%s%lld bytes of shared memory)"); \
     int per_sm = 1;                                                                                    \
     MCRE_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, threads, smem));               \
     if (per_sm < 1) return fail(-3, "irc main kernel does not fit: too many metric dates x tangents%s", ""); \

@@ -60,11 +60,11 @@ __global__ void irc_patch_coefficients_kernel(const double *__restrict__ coef, i
       if (e >= 0) {
         const double *dr = date_rec + (size_t)di * DR;
         const double sh = dr[4], sc = dr[5];
-        const double c0 = coef[(size_t)e * 3], c1 = coef[(size_t)e * 3 + 1], c2 = coef[(size_t)e * 3 + 2];
-        // c(u), u = (r - shift) scale  ->  c'(r) in the raw basis [1, r, r^2]
-        r[12] = g * (c2 * sc * sc);
-        r[11] = g * (c1 * sc - 2.0 * c2 * sc * sc * sh);
-        r[10] = g * (c0 - c1 * sc * sh + c2 * sc * sc * sh * sh);
+        double raw[3];
+        irc_raw_basis(coef[(size_t)e * 3], coef[(size_t)e * 3 + 1], coef[(size_t)e * 3 + 2], sh, sc, raw);
+        r[12] = __dmul_rn(g, raw[2]);
+        r[11] = __dmul_rn(g, raw[1]);
+        r[10] = __dmul_rn(g, raw[0]);
       }
     }
   }

@@ -351,6 +351,16 @@ static int launch_forward_tan(const IrcDev &d, const RngDev &r, const ShardDev &
   return 0;
 }
 
+static size_t tangent_moments_smem(const IrcDev &d) { return ((size_t)d.n_reg * TM_NV + 2 * (256 / 32) * TM_NV) * sizeof(double); }
+
+// Checks that the tangent moments kernel fits the plan's regression dates (and requests its shared memory); called by
+// mcre_irc_presim before anything is launched.
+int irc_presim_tangent_fit(const mcre_irc_plan *p) {
+  MCRE_SMEM(irc_presim_tangent_moments_kernel, tangent_moments_smem(p->d),
+            "irc tangent presim kernel does not fit: too many regression dates (%s%lld bytes of shared memory)");
+  return 0;
+}
+
 // Forward pass with tangents + tangent moments; the value moments of the same scratch are
 // accumulated by mcre_irc_presim (which calls this first when the plan carries tangents).
 int irc_presim_tangent_pass(mcre_irc_plan *p, const RngDev &r, const ShardDev &sh, void *d_scratch, double *d_partial,
@@ -367,11 +377,10 @@ int irc_presim_tangent_pass(mcre_irc_plan *p, const RngDev &r, const ShardDev &s
   int rc = d.nt == 4 ? launch_forward_tan<4>(d, r, sh, xbuf, nbuf, wbuf, dx, dn, dw, st)
                      : launch_forward_tan<8>(d, r, sh, xbuf, nbuf, wbuf, dx, dn, dw, st);
   if (rc) return rc;
-  const int threads = 256, nw = threads / 32;
-  const size_t smem = ((size_t)d.n_reg * TM_NV + 2 * nw * TM_NV) * sizeof(double);
+  const int threads = 256;
+  const size_t smem = tangent_moments_smem(d);
   const long long n_chunks = (n + sh.chunk - 1) / sh.chunk;
   auto k = irc_presim_tangent_moments_kernel;
-  if (smem > 32 * 1024) MCRE_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   int per_sm = 1;
   MCRE_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, threads, smem));
   if (per_sm < 1) return fail(-3, "irc tangent presim kernel does not fit: too many regression dates%s", "");

@@ -325,7 +325,7 @@ static int launch_value(mcre_irc_plan *p, const RngDev &rng, const ShardDev &sh,
 #define LAUNCHV(CIRV)                                                                                     \
   do {                                                                                                    \
     auto k = irc_value_kernel<NS, CIRV>;                                                                  \
-    if (smem > 32 * 1024) MCRE_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+    MCRE_SMEM(k, smem, "irc value kernel does not fit: too many metric dates / too long an MPoR look-back (%s%lld bytes of shared memory)"); \
     int per_sm = 1;                                                                                       \
     MCRE_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, 128, smem));                      \
     if (per_sm < 1) return fail(-3, "irc value kernel does not fit: too many metric dates / too long an MPoR look-back%s", "");        \

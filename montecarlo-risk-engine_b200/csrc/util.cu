@@ -23,6 +23,17 @@ int sm_count() {
   return cached;
 }
 
+int smem_optin_limit() {
+  static int cached = 0;
+  if (cached == 0) {
+    int dev = 0;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&cached, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
+    if (cached <= 0) cached = 48 * 1024;
+  }
+  return cached;
+}
+
 // Balanced pairwise sum over chunks, defined by a binary-counter stack: element i is pushed at
 // level 0 and equal-level neighbours are merged immediately; leftover levels (non power-of-two
 // counts) fold from the most recent to the oldest.  For a power-of-two count this is exactly the
