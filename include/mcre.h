@@ -644,6 +644,7 @@ int mcre_correlated_normals(const mcre_rng *rng, int32_t n_sub, int32_t dim, con
 #define MCRE_STORAGE_STEP 24       /* doubles per sub-step record                                       */
 #define MCRE_STORAGE_MAX_NOISE 8   /* normals per sub-step of the price model's joint draw              */
 #define MCRE_STORAGE_MAX_BASIS 6   /* regression basis functions (polynomial degree + 1)                */
+#define MCRE_STORAGE_TAN 7         /* doubles per (sub-step, tangent slot) record of step_tan           */
 
 typedef struct {
   int32_t n_sub;            /* sub-steps of the simulation grid (engine.py:36-123)                         */
@@ -675,11 +676,16 @@ typedef struct {
   const double *numeraire;  /* [n_dates] numeraire at the action dates                                     */
   int32_t noise_dim;        /* normals per sub-step of the model's joint draw: 2 (Schwartz two-factor), 1 (Black-Scholes),
                                number of assets (Black-Scholes multi-asset), <= MCRE_STORAGE_MAX_NOISE         */
-  int32_t n_tan;            /* 0, or 3 / 6: pathwise PV sensitivities with respect to that many model parameters   */
-  const double *step_tan;   /* [n_sub][n_tan][6] d(A, B00, M, B10, B11, log F)/d parameter of the effective recursion
-                               x' = A x + B00 z0, y' = y + M + B10 z0 + B11 z1 (A = a - k dt, B00 = cx bx_0, B10 = cy by_0,
-                               B11 = cy by_1; noise_dim <= 2); entry [0][.][5] also holds d log F(t0)           */
-  const double *dlog_num;   /* [n_dates][n_tan] d log numeraire / d parameter                                  */
+  int32_t n_tan;            /* 0, or 3 / 4 / 6: pathwise PV sensitivities with respect to that many tangent slots of
+                               the storage (spot, volatility, rate of a Black-Scholes asset [, rate of the numeraire
+                               model]; the six Schwartz parameters), which the caller maps to the model's parameters */
+  const double *step_tan;   /* [n_sub][n_tan][MCRE_STORAGE_TAN] d(A, B00, M, B10, B11, log F, Bw)/d slot of the effective
+                               recursion x' = A x + B00 z0, y' = y + M + B10 z0 + B11 z1 (A = a - k dt, B00 = cx bx_0,
+                               B10 = cy by_0, B11 = cy by_1), where d(cx w0) also gains dBw w0 (Bw: d log of the asset's
+                               row of the joint Cholesky factor; 0 for the one- and two-factor stand-alone steps);
+                               Black-Scholes EULER steps: dx' = dx + (dM + dBw w0) / (1 + m + cx w0) with dM = d m,
+                               dBw = d cx; entry [0][.][5] also holds d log F(t0)                                */
+  const double *dlog_num;   /* [n_dates][n_tan] d log numeraire / d slot                                        */
   /* ---- exposure dates (controller.py:412-447); n_expo = 0: none ---- */
   int32_t n_expo;           /* internal exposure dates                                                         */
   int32_t n_pre_expo;       /* leading exposure dates at the calibration date                                  */

@@ -33,9 +33,10 @@ struct StorageDev {
   const int *step_date;     // [n_sub]
   const double *rec;        // [n_dates][ST_REC]
   const double *numeraire;  // [n_dates]
-  // pathwise PV sensitivities (n_tan > 0): tangents of the effective linear recursion per sub-step and parameter,
-  // [n_sub][n_tan][6] = d(A, B00, M, B10, B11, log F) with x' = A x + B00 z0, y' = y + M + B10 z0 + B11 z1, and
-  // d log numeraire / d parameter per action date [n_dates][n_tan]
+  // pathwise PV sensitivities (n_tan > 0) with respect to the storage's own tangent slots (the host scatters them into
+  // the model's flattened parameters): tangents of the effective recursion per sub-step and slot, [n_sub][n_tan][ST_TAN]
+  // = d(A, B00, M, B10, B11, log F, Bw) with x' = A x + B00 z0 + Bw-scaled w0, y' = y + M + B10 z0 + B11 z1 (see
+  // storage_main_kernel), and d log numeraire / d slot per action date [n_dates][n_tan]
   int noise_dim, n_tan;
   const double *step_tan, *dlog_num;
   // exposure dates (controller.py:412-447): n_expo internal exposure dates, the first n_pre_expo at the calibration date;
@@ -144,6 +145,7 @@ __device__ __forceinline__ int best_of(const double (&v)[3]) {
 // [8 + j] bx_j, [16 + j] by_j.
 constexpr int ST_STEP = MCRE_STORAGE_STEP;
 constexpr int ST_NOISE = MCRE_STORAGE_MAX_NOISE;
+constexpr int ST_TAN = MCRE_STORAGE_TAN;
 struct TwoFactor {
   double x = 0.0, y = 0.0;
   __device__ __forceinline__ double advance(const double *__restrict__ st, double w0, double w1) {
@@ -465,7 +467,14 @@ __global__ void __launch_bounds__(32) storage_solve_kernel(int S, int NB, const 
 // NT > 0: pathwise sensitivities of the PV with respect to the NT model parameters, the way the reference's autograd sees
 // them (controller.py:609-627): the arg-max and the inventory moves carry no gradient, a cashflow
 // -dV (S +- cost) / N differentiates to -dV dS / N - cashflow dlogN, and dS = S dlogS follows the tangent recursion of
-// the factors.  Per-path tangents are ADDED to tan [NT][n_paths].
+// the factors:
+//   two-factor step     dx' = A dx + dA x + dB00 z0 + dBw w0,  dy' = dy + dM + dB10 z0 + dB11 z1
+//                       (dBw w0 = d(sum_j bx_j z_j): a Black-Scholes asset of a joint draw, whose row of the Cholesky
+//                       factor of D C D dt is proportional to its own volatility; 0 for the other models)
+//   Black-Scholes EULER dx' = dx + (dM + dBw w0) / (1 + m + cx w0)   (dM = d(rate dt), dBw = d(sigma sqrt(dt)))
+// NT counts the storage's own tangent slots (3: spot, volatility, rate of a Black-Scholes asset, + 1: the numeraire
+// model's rate; 6: the Schwartz parameters), not the parameters of the joint model.
+// Per-path tangents are ADDED to tan [NT][n_paths].
 template <int NT>
 __global__ void __launch_bounds__(ST_THREADS) storage_main_kernel(StorageDev P, RngDev rng, long long path_begin,
                                                                   long long n_paths, const double *__restrict__ coef,
@@ -539,7 +548,7 @@ __global__ void __launch_bounds__(ST_THREADS) storage_main_kernel(StorageDev P, 
     // its tangent is stored with the first sub-step
     if (P.n_sub > 0) {
 #pragma unroll
-      for (int k = 0; k < NT; ++k) dls[k] = __ldg(P.step_tan + (size_t)k * 6 + 5);
+      for (int k = 0; k < NT; ++k) dls[k] = __ldg(P.step_tan + (size_t)k * ST_TAN + 5);
     }
   }
   for (int d = 0; d < P.n_pre_dates; ++d) act(d, s0);
@@ -552,14 +561,25 @@ __global__ void __launch_bounds__(ST_THREADS) storage_main_kernel(StorageDev P, 
     draw_w(rng, ns, P.noise_dim, is, gp, st, w0, w1, z0, z1);
     const double ls = f.advance(st, w0, w1);
     if constexpr (NT > 0) {
-      const double A = __ldg(st + 0) - __ldg(st + 1) * __ldg(st + 2);
-      const double *tt = P.step_tan + (size_t)is * NT * 6;
+      const double *tt = P.step_tan + (size_t)is * NT * ST_TAN;
+      if (__ldg(st + 7) != 0.0) {
+        const double inv = 1.0 / (1.0 + __dadd_rn(__ldg(st + 3), __dmul_rn(__ldg(st + 4), w0)));
 #pragma unroll
-      for (int k = 0; k < NT; ++k) {
-        const double *t6 = tt + k * 6;
-        dx[k] = A * dx[k] + __ldg(t6 + 0) * x_old + __ldg(t6 + 1) * z0;
-        dy[k] = dy[k] + __ldg(t6 + 2) + __ldg(t6 + 3) * z0 + __ldg(t6 + 4) * z1;
-        dls[k] = __ldg(t6 + 5) + dx[k] + dy[k];
+        for (int k = 0; k < NT; ++k) {
+          const double *t7 = tt + k * ST_TAN;
+          dx[k] = dx[k] + (__ldg(t7 + 2) + __ldg(t7 + 6) * w0) * inv;
+          dls[k] = __ldg(t7 + 5) + dx[k];
+        }
+      } else {
+        const double A = __ldg(st + 0) - __ldg(st + 1) * __ldg(st + 2);
+#pragma unroll
+        for (int k = 0; k < NT; ++k) {
+          const double *t7 = tt + k * ST_TAN;
+          dx[k] = A * dx[k] + __ldg(t7 + 0) * x_old + __ldg(t7 + 1) * z0;
+          dx[k] = fma(__ldg(t7 + 6), w0, dx[k]);
+          dy[k] = dy[k] + __ldg(t7 + 2) + __ldg(t7 + 3) * z0 + __ldg(t7 + 4) * z1;
+          dls[k] = __ldg(t7 + 5) + dx[k] + dy[k];
+        }
       }
     }
     const int d = __ldg(P.step_date + is);
@@ -587,8 +607,8 @@ extern "C" int mcre_storage_create(const mcre_storage_desc *c, mcre_storage_plan
   if (c->n_states < 2 || c->n_states > ST_MAX_S) return fail(-2, "storage: 2..%s%lld inventory states", "", ST_MAX_S);
   if (c->n_basis < 1 || c->n_basis > ST_MAX_B) return fail(-2, "storage: 1..%s%lld basis functions", "", ST_MAX_B);
   if (c->noise_dim < 1 || c->noise_dim > ST_NOISE) return fail(-2, "storage: 1..8 noise factors%s", "");
-  if (c->n_tan > 0 && c->noise_dim > 2) return fail(-3, "storage: sensitivities for one- and two-factor price models%s", "");
-  if (c->n_tan != 0 && c->n_tan != 3 && c->n_tan != 6) return fail(-2, "storage: 0, 3 or 6 tangent directions%s", "");
+  if (c->n_tan != 0 && c->n_tan != 3 && c->n_tan != 4 && c->n_tan != 6)
+    return fail(-2, "storage: 0, 3, 4 or 6 tangent directions%s", "");
   if (c->n_tan > 0 && (!c->step_tan || !c->dlog_num)) return fail(-1, "storage: tangent tables missing%s", "");
   if (c->n_expo < 0 || c->n_pre_expo < 0 || c->n_pre_expo > c->n_expo || (c->n_expo > 0 && (!c->expo_numeraire || (c->n_sub > 0 && !c->step_expo))))
     return fail(-2, "storage: bad exposure tables%s", "");
@@ -608,7 +628,7 @@ extern "C" int mcre_storage_create(const mcre_storage_desc *c, mcre_storage_plan
     if (!rc) rc = p->numeraire.upload(c->numeraire, (size_t)c->n_dates);
     if (!rc && c->n_expo > 0) rc = p->step_expo.upload(c->step_expo, (size_t)c->n_sub);
     if (!rc && c->n_expo > 0) rc = p->expo_num.upload(c->expo_numeraire, (size_t)c->n_expo);
-    if (!rc && c->n_tan > 0) rc = p->step_tan.upload(c->step_tan, (size_t)c->n_sub * c->n_tan * 6);
+    if (!rc && c->n_tan > 0) rc = p->step_tan.upload(c->step_tan, (size_t)c->n_sub * c->n_tan * ST_TAN);
     if (!rc && c->n_tan > 0) rc = p->dlog_num.upload(c->dlog_num, (size_t)c->n_dates * c->n_tan);
     if (!rc) rc = p->arena.commit();
   }
@@ -702,6 +722,7 @@ extern "C" int mcre_storage_mainsim(mcre_storage_plan *p, const mcre_rng *rng, c
                                                                      initial_state, d_cfs, d_final_state, d_tan, d_coef_expo, d_expo)
   if (p->d.n_tan == 0) GO(0);
   else if (p->d.n_tan == 3) GO(3);
+  else if (p->d.n_tan == 4) GO(4);
   else GO(6);
 #undef GO
   MCRE_LAUNCHED();

@@ -42,6 +42,7 @@ from mcre.timegrid import build_time_grid
 LAPACK_MAX_PATHS = 1 << 16
 STEP = 24
 MAX_NOISE = 8
+TAN = 7
 
 
 def _is_storage(p):
@@ -79,36 +80,70 @@ def rate_of(model):
     return model.param_values()[2 * model.num_assets if _is_bsm(model) else (2 if _is_bs(model) else 0)]
 
 
-def step_table(model, grid, scheme, nt=0, asset_id=None):
-    """-> (steps [n_sub][STEP], tangents [n_sub][nt][6] or None): records of csrc/storage.cu:TwoFactor and, for pathwise
-    sensitivities, d(A, B00, M, B10, B11, log F) / d(parameter) of the effective recursion x' = A x + B00 z0,
-    y' = y + M + B10 z0 + B11 z1 (host duals, mcre/dual.py; one- and two-factor models).
+def tangent_slots(model, asset_id=None):
+    """-> (slots, numeraire slot): the flattened parameter index of each tangent slot of a storage on `asset_id`, and the
+    slot of the numeraire model's rate.  The slots are the parameters the storage's step depends on - the lane
+    parameters of mcre/equity.py:family_of (spot, volatility, rate of a Black-Scholes asset; the six Schwartz
+    parameters) - and, when the numeraire is another model of a ModelConfig, that model's rate (its discount factors)."""
+    from mcre.equity import EquityBackend, family_of
+    from models.model_config import ModelConfig
+    fam = family_of(model)
+    if fam is None:
+        raise NotImplementedError("gas storage: sensitivities on Schwartz two-factor, Black-Scholes and Black-Scholes "
+                                  "multi-asset models, or a ModelConfig of Black-Scholes models")
+    _, assets = fam
+    asset = assets[0] if len(assets) == 1 else next(a for a in assets if a.asset_id == asset_id)
+    if isinstance(model, ModelConfig):
+        num_idx = model.id_to_model["numeraire"]
+        num_global = model.param_offsets()[num_idx] + EquityBackend._rate_index(model.models[num_idx])
+    else:
+        num_global = EquityBackend._rate_index(model)
+    slots = list(asset.gmap)
+    if num_global not in slots:
+        slots.append(num_global)
+    return slots, slots.index(num_global)
+
+
+def step_table(model, grid, scheme, nt=0, asset_id=None, kernel_record=False):
+    """-> (steps [n_sub][STEP], tangents [n_sub][nt][6] or None): records of csrc/storage.cu:TwoFactor and, for
+    pathwise sensitivities, d(A, B00, M, B10, B11, log F) / d(slot) of the effective recursion x' = A x + B00 z0,
+    y' = y + M + B10 z0 + B11 z1, or of the Black-Scholes EULER step (host duals, mcre/dual.py); kernel_record: the
+    kernel's [n_sub][nt][TAN] records, which also hold d Bw, the tangent that scales the combined draw w0.  The
+    slots are the storage's own (tangent_slots): nt = 6 Schwartz parameters, or 3 (spot, volatility, rate of the asset's
+    model) + an optional 4th, the numeraire model's rate, on which no step depends.
     Schwartz two-factor (schwartz_two_factor.py:124-196), parameters [rate, kappa, sigma_s, mu_l, sigma_l, rho]:
       ANALYTICAL  a = exp(-kappa dt), b = Cholesky factor of the step covariance (cached per nominal dt, model.py:45-64)
       EULER       a = 1, k = kappa, cx / cy = sigma sqrt(dt), b = Cholesky factor of the correlation - which the
                   reference builds before requires_grad(): rho is a constant of its autograd graph there
-    Black-Scholes (black_scholes.py:50-67, ANALYTICAL only; parameters [spot, sigma, rate]): the log-price accumulates in
+    Black-Scholes (black_scholes.py:50-67, parameters [spot, sigma, rate]), ANALYTICAL: the log-price accumulates in
     x (bx_0 = sqrt(sigma^2 dt)), its drift (rate - sigma^2 / 2) dt in m, log F = log spot.
-    Black-Scholes multi-asset (black_scholes_multi.py:63-79, ANALYTICAL, value-only): the same for the asset `asset_id`
-    with bx = its row of the Cholesky factor of the step covariance of all assets - the draw is the model's joint one."""
+    Black-Scholes multi-asset (black_scholes_multi.py:63-79) or a Black-Scholes model of a ModelConfig, ANALYTICAL: the
+    same for the asset `asset_id` with bx = its row of the Cholesky factor of the step covariance D C D dt of all assets
+    - the draw is the model's joint one.  That row is sigma_a sqrt(dt) L_C[a, :], so d bx = bx d log sigma_a: the
+    tangent multiplies the combined draw w0 (Bw = log sigma_a), and the other assets' volatilities do not reach it.
+    EULER (black_scholes.py:69-85, black_scholes_multi.py:81-97): x' = x + log1p(m + cx w0), m = rate dt,
+    cx = sigma sqrt(dt), bx = the asset's row of the Cholesky factor of the correlation (a constant); the tangent record
+    holds dM = d m, dBw = d cx and d log F."""
     from mcre.dual import D, dexp, dlog, dsqrt
-    from models.model_config import ModelConfig
     joint = model
     model, noise_off, noise_dim, _ = price_model_of(joint, asset_id)
     if noise_dim > MAX_NOISE:
         raise NotImplementedError(f"gas storage: price models with at most {MAX_NOISE} noise factors")
-    if nt and joint is not model:
-        raise NotImplementedError("gas storage: sensitivities on a stand-alone price model")
-    p = model.dual_params(0, nt)
     zero, one = D(0.0, None, nt), D(1.0, None, nt)
     out = np.zeros((max(grid.n_sub, 1), STEP))
-    tan = np.zeros((max(grid.n_sub, 1), nt, 6)) if nt else None
+    tan = np.zeros((max(grid.n_sub, 1), nt, TAN)) if nt else None
     chol = {}
     black_scholes = _is_bs(model) or _is_bsm(model)
+    if black_scholes:
+        n = model.num_assets if _is_bsm(model) else 1
+        ai = model.asset_ids.index(asset_id) if _is_bsm(model) else 0
+        vals = model.param_values()
+        # (slots 0, 1, 2: spot, volatility, rate of the asset; the same order as dual_params of a BlackScholesModel)
+        spot, sig, rate = [D.var(v, k, nt) if nt else D(v, None, 0) for k, v in enumerate((vals[ai], vals[n + ai], vals[2 * n]))]
+    else:
+        p = model.dual_params(0, nt)
     if black_scholes and scheme not in (SimulationScheme.ANALYTICAL, SimulationScheme.EULER):
         raise NotImplementedError(f"gas storage on Black-Scholes models: scheme {scheme}")
-    if black_scholes and scheme == SimulationScheme.EULER and nt:
-        raise NotImplementedError("gas storage: sensitivities under the ANALYTICAL scheme for Black-Scholes price models")
 
     def joint_factor(key):
         """Lower Cholesky factor of the joint step covariance (ANALYTICAL) / correlation (EULER) of the whole draw
@@ -120,11 +155,9 @@ def step_table(model, grid, scheme, nt=0, asset_id=None):
     for s in range(grid.n_sub):
         dt = grid.dt[s]
         bx, by = [zero] * MAX_NOISE, [zero] * MAX_NOISE
+        bw = zero
         euler_bs = 0.0
         if black_scholes:
-            n = model.num_assets if _is_bsm(model) else 1
-            ai = model.asset_ids.index(asset_id) if _is_bsm(model) else 0
-            spot, sig, rate = (p[ai], p[n + ai], p[2 * n]) if _is_bsm(model) else p
             col = noise_off + ai
             a, k, cx, cy, lf = one, zero, one, zero, dlog(spot)
             if scheme == SimulationScheme.EULER:
@@ -139,6 +172,7 @@ def step_table(model, grid, scheme, nt=0, asset_id=None):
                 L = joint_factor(grid.dt_nominal[s])
                 m = (rate - 0.5 * sig * sig) * dt if _is_bsm(model) else rate * dt - 0.5 * dt * sig * sig
                 bx = [D(float(L[col, j]), None, nt) if j <= col else zero for j in range(MAX_NOISE)]
+                bw = dlog(sig)
         else:
             rate, kappa, sig_s, mu, sig_l, rho = p
             if scheme == SimulationScheme.ANALYTICAL:
@@ -173,10 +207,13 @@ def step_table(model, grid, scheme, nt=0, asset_id=None):
         out[s, 8:8 + MAX_NOISE] = [val(x) for x in bx]
         out[s, 16:16 + MAX_NOISE] = [val(x) for x in by]
         if nt:
-            eff = (a - k * dt, cx * bx[0], m, cy * by[0], cy * by[1], lf)
+            if euler_bs:
+                eff = (zero, zero, m, zero, zero, lf, cx)
+            else:
+                eff = (a - k * dt, cx * bx[0], m, cy * by[0], cy * by[1], lf, bw)
             for j, e in enumerate(eff):
                 tan[s, :, j] = D.lift(e, nt).t
-    return out, tan
+    return out, (tan if tan is None or kernel_record else tan[:, :, :6])
 
 
 def log_spot_scale(model, t):
@@ -227,16 +264,23 @@ class StorageBackend:
             raise NotImplementedError("gas storage: CVA of a book of storages alone (the default weights ride with an equity "
                                       "launch of the same netting set)")
         self.need_expo = c.risk_metrics.requires_exposure_profiles()
-        if c.differentiate and (self.mixed or not self.standalone or _is_bsm(c.model) or self.need_expo):
-            raise NotImplementedError("gas storage: sensitivities of the PV of books of storages on a one- or two-factor "
-                                      "price model")
-        self.nt = len(c.model.model_params) if c.differentiate else 0
+        if c.differentiate and self.need_expo:
+            raise NotImplementedError("gas storage: sensitivities of exposure metrics and CVA (PV sensitivities only)")
+        if c.differentiate and any(isinstance(m, CIRPPModel) for m in subs):
+            raise NotImplementedError("gas storage: sensitivities in a ModelConfig with a credit model")
         for p in c.products:
             if _is_storage(p):
                 price_model_of(c.model, p.get_asset_id())      # raises for an unknown asset id
         num_model = price_model_of(c.model, [p for p in c.products if _is_storage(p)][0].get_asset_id())[3]
         self.num_rate = rate_of(num_model)
-        self.rate_index = 2 if _is_bs(c.model) else 0           # (tangent slot of the rate: stand-alone one- / two-factor models)
+        #: tangent slots of each storage (tangent_slots): asset id -> (flattened parameter index per slot, numeraire slot)
+        self.slots = {}
+        if c.differentiate:
+            for p in c.products:
+                if _is_storage(p) and p.get_asset_id() not in self.slots:
+                    self.slots[p.get_asset_id()] = tangent_slots(c.model, p.get_asset_id())
+        #: tangent slots per storage lane (csrc/storage.cu:storage_main_kernel<NT>); 0: values only
+        self.nt = max(len(g) for g, _ in self.slots.values()) if self.slots else 0
         self.noise_dim = int(c.model.simulation_dim)
         if self.noise_dim > MAX_NOISE:
             raise NotImplementedError(f"gas storage: price models with at most {MAX_NOISE} noise factors")
@@ -270,15 +314,17 @@ class StorageBackend:
         t0 = self._t0()
         rate = self.num_rate
         numeraire = np.array([math.exp(rate * (t - t0)) for t in acts])
-        dlog_num = np.zeros((len(acts), max(self.nt, 1)))
-        if self.nt:
-            dlog_num[:, self.rate_index] = [t - t0 for t in acts]
+        slots, num_slot = self.slots.get(prod.get_asset_id(), ([], 0))
+        nt = len(slots)
+        dlog_num = np.zeros((len(acts), max(nt, 1)))
+        if nt:
+            dlog_num[:, num_slot] = [t - t0 for t in acts]
         keep = []
         d = B.StorageDesc()
         d.n_sub, d.n_dates, d.n_pre_dates = grid.n_sub, len(acts), n_pre
         d.n_states, d.n_basis = prod.num_states, self.n_basis
         d.log_spot0 = math.log(self._spot0(prod))
-        d.noise_dim, d.n_tan = self.noise_dim, self.nt
+        d.noise_dim, d.n_tan = self.noise_dim, nt
         expo_times = c.exposure_timeline.tolist() if self.need_expo else []
         for t in expo_times:
             # two dates one rounding error apart share a simulation date; the kernel acts before it reads the exposure of
@@ -292,7 +338,7 @@ class StorageBackend:
         expo_num = np.array([math.exp(rate * (t - t0)) for t in expo_times]) if expo_times else np.zeros(1)
         for name, arr, conv in (("step_expo", step_expo if (grid.n_sub and expo_times) else np.zeros(1, np.int32), B.as_ip),
                                 ("expo_numeraire", expo_num, B.as_dp),
-                                ("step_tan", steps_tan if self.nt else np.zeros(1), B.as_dp), ("dlog_num", dlog_num, B.as_dp),
+                                ("step_tan", steps_tan if nt else np.zeros(1), B.as_dp), ("dlog_num", dlog_num, B.as_dp),
                                 ("step", steps, B.as_dp), ("step_date", step_date if grid.n_sub else np.zeros(1, np.int32), B.as_ip),
                                 ("date_rec", rec, B.as_dp), ("numeraire", numeraire, B.as_dp)):
             a, ptr = conv(arr)
@@ -428,7 +474,8 @@ class StorageBackend:
         def steps_of(prod):
             key = None if (self.standalone and not _is_bsm(c.model)) else prod.get_asset_id()
             if key not in step_cache:
-                step_cache[key] = step_table(c.model, grid, c.simulation_scheme, self.nt, asset_id=key)
+                nt = len(self.slots[prod.get_asset_id()][0]) if self.nt else 0
+                step_cache[key] = step_table(c.model, grid, c.simulation_scheme, nt, asset_id=key, kernel_record=True)
             return step_cache[key]
         n_main = c.num_paths_mainsim
         if self.mixed or self.need_expo:
@@ -444,8 +491,9 @@ class StorageBackend:
         n_expo = len(c.exposure_timeline) if self.need_expo else 0
         expos = [torch.zeros((n_expo, max(count, 1)), dtype=torch.float64, device=dev) if n_expo else None
                  for _ in c.netting_sets]
-        tans = [torch.zeros((self.nt, max(count, 1)), dtype=torch.float64, device=dev) if self.nt else None
-                for _ in c.netting_sets]
+        # per-path tangents, one buffer per (netting set, tangent slots): the storages of a set that share their slots add
+        # into one buffer, whose fixed-order chunk sums are scattered into the set's gradient at the end
+        tans = [{} for _ in c.netting_sets]
         try:
             for pi, prod in enumerate(c.products):
                 if not _is_storage(prod):
@@ -457,16 +505,23 @@ class StorageBackend:
                 torch.cuda.current_stream().synchronize()
                 t_pre += time.perf_counter() - t0
                 si = c.product_to_netting_set_idx[pi]
+                tan = None
+                if self.nt:
+                    key = tuple(self.slots[prod.get_asset_id()][0])
+                    if key not in tans[si]:
+                        tans[si][key] = torch.zeros((len(key), max(count, 1)), dtype=torch.float64, device=dev)
+                    tan = tans[si][key]
                 B.check(L.mcre_storage_mainsim(plan, C.byref(rng_main), C.byref(shard), coef.data_ptr(),
                                                float(prod.get_initial_state()), cfs[si].data_ptr(), None,
-                                               tans[si].data_ptr() if self.nt else None,
+                                               tan.data_ptr() if self.nt else None,
                                                coef_e.data_ptr() if n_expo else None,
                                                expos[si].data_ptr() if n_expo else None, RT.stream_ptr()))
-            if self.mixed or self.need_expo:
-                return self._finish_mixed(cfs, expos, chunk, dev, t_start, t_pre)
-            raw = []
             n_chunks = max((count + chunk - 1) // chunk, 1)
             partial = torch.empty(n_chunks * 2 * max(self.nt, 1) + 1, dtype=torch.float64, device=dev)
+            grads = [self._gradient(t, count, chunk, partial, dev) for t in tans] if self.nt else None
+            if self.mixed or self.need_expo:
+                return self._finish_mixed(cfs, expos, grads, chunk, dev, t_start, t_pre)
+            raw = []
             unconnected = c.model.unconnected_params(c.simulation_scheme)
             used = [i not in unconnected for i in range(len(c.model.model_params))]
             for si in range(len(c.netting_sets)):
@@ -478,15 +533,7 @@ class StorageBackend:
                                          out.data_ptr(), RT.stream_ptr()))
                 s = RT.to_host(RT.all_reduce_tree(out))
                 pv = mean_and_error(float(s[0]), float(s[1]), float(RT.to_host(shift)[0]), n_main)
-                grad = None
-                if self.nt:
-                    # sums of the per-path tangents in the same fixed chunk order (shift 0); mean = sum / n
-                    zero = torch.zeros(self.nt, dtype=torch.float64, device=dev)
-                    out_t = torch.zeros(self.nt * 2, dtype=torch.float64, device=dev)
-                    B.check(L.mcre_sum_stats(tans[si].data_ptr(), count, self.nt, chunk, zero.data_ptr(), 0,
-                                             partial.data_ptr(), out_t.data_ptr(), RT.stream_ptr()))
-                    grad = RT.to_host(RT.all_reduce_tree(out_t)).reshape(self.nt, 2)[:, 0] / n_main
-                raw.append({"pv": (pv, grad), "param_used": lambda kind: used})
+                raw.append({"pv": (pv, grads[si] if self.nt else None), "param_used": lambda kind: used})
         finally:
             torch.cuda.current_stream().synchronize()
             for plan in plans:
@@ -495,10 +542,27 @@ class StorageBackend:
         return raw, {"preprocessing": t_pre, "path_generation": total - t_pre, "request_resolution": 0.0}
 
 
-    def _finish_mixed(self, cfs, expos, chunk, dev, t_start, t_pre):
+    def _gradient(self, tans, count, chunk, partial, dev):
+        """PV gradient [n_params] of one netting set's storages: the sums of the per-path tangents of each buffer
+        {slots: [len(slots)][count]} in the fixed chunk order of mcre_sum_stats (shift 0) and the rank tree - the same
+        bits on any number of GPUs - over the path count, scattered to the slots' parameters."""
+        L = B.lib()
+        grad = np.zeros(len(self.c.model.model_params))
+        for slots, tan in tans.items():
+            nt = len(slots)
+            zero = torch.zeros(nt, dtype=torch.float64, device=dev)
+            out_t = torch.zeros(nt * 2, dtype=torch.float64, device=dev)
+            B.check(L.mcre_sum_stats(tan.data_ptr(), count, nt, chunk, zero.data_ptr(), 0, partial.data_ptr(),
+                                     out_t.data_ptr(), RT.stream_ptr()))
+            grad[list(slots)] += RT.to_host(RT.all_reduce_tree(out_t)).reshape(nt, 2)[:, 0] / self.c.num_paths_mainsim
+        return grad
+
+    def _finish_mixed(self, cfs, expos, grads, chunk, dev, t_start, t_pre):
         """The other products of the run through the equity backend's accumulating launches, starting from the
         storages' per-path discounted cashflows and exposures (same Philox streams: the draw is the model's joint one);
-        that path also applies threshold / collateral and finishes EPE / ENE / PFE - for books of storages alone, too."""
+        that path also applies threshold / collateral and finishes EPE / ENE / PFE - for books of storages alone, too.
+        With sensitivities (PV only) the equity launches run with tangents, and a set's gradient is theirs plus the
+        storages' `grads`."""
         import copy
         from mcre.equity import EquityBackend, is_equity_exercise
         c = self.c
@@ -525,6 +589,9 @@ class StorageBackend:
         for si in range(len(c.netting_sets)):
             res = eb._run_split_book(si, dev, c.num_paths_mainsim, n_params, chunk=chunk, extra_pv=cfs[si],
                                      extra_expo=expos[si])
+            if grads is not None:
+                pv, grad = res["pv"]
+                res["pv"] = (pv, grad + grads[si])
             raw.append(res)
         torch.cuda.synchronize(dev)
         total = time.perf_counter() - t_start

@@ -5,7 +5,7 @@ Americans, FlexiCalls and gas storages in ONE netting set, PV metric, 1000 paths
 The path-dependent / exercise products exceed what one launch tracks, so the book is split over launches
 (mcre/equity.py:_run_split_book).
 
-    python tools/large_book.py [--scale 1.0] [--paths 1000]
+    python tools/large_book.py [--scale 1.0] [--paths 1000] [--differentiate]
 """
 import argparse
 import importlib
@@ -77,7 +77,12 @@ def main():
     ap.add_argument("--cva", action="store_true",
                     help="CVA of the book against a counterparty with a CIR++ intensity, 80 exposure dates over the book's "
                          "horizon, MPoR 10 days, EULER (tests/exposure_tests/cva_perfprmance_large_netting_set.py:69-193)")
+    ap.add_argument("--differentiate", action="store_true",
+                    help="PV with first-order pathwise sensitivities to every model parameter; also prints the norm of the "
+                         "gradient and the number of derivatives that are not None")
     args = ap.parse_args()
+    if args.differentiate and (args.cva or args.exposure_points > 0):
+        ap.error("--differentiate runs the PV book")
     importlib.import_module("montecarlo-risk-engine_b200")
     import torch
     import cases
@@ -109,11 +114,11 @@ def main():
         rm = ns.RiskMetrics([ns.EPEMetric(), ns.PFEMetric(0.95)], exposure_timeline=np.linspace(0.0, 2.5, args.exposure_points))
     else:
         rm = ns.RiskMetrics([ns.PVMetric()])
-    sc = ns.SimulationController([nset], model, rm, args.paths, args.paths, 1, scheme, False)
+    sc = ns.SimulationController([nset], model, rm, args.paths, args.paths, 1, scheme, args.differentiate)
     # warm-up on a tiny book of the same kinds: CUDA module loading and allocator growth are not product work
     warm = build_book(ns, ids, {k: 2 for k in base})
     ns.SimulationController([ns.NettingSet(name="warm", products=warm)], model, ns.RiskMetrics([ns.PVMetric()]), args.paths,
-                            args.paths, 1, scheme, False).run_simulation()
+                            args.paths, 1, scheme, args.differentiate).run_simulation()
     torch.cuda.synchronize()
     l0 = B.launch_count()
     t0 = time.perf_counter()
@@ -131,6 +136,9 @@ def main():
     else:
         shown = {"pv": float(res.get_results(nset.get_name(), "pv", evaluation_idx=0)),
                  "mc_error": float(res.get_mc_error(nset.get_name(), "pv", evaluation_idx=0))}
+        if args.differentiate:
+            grad = [g for g in res.get_derivatives(nset.get_name(), "pv")[0] if g is not None]
+            shown.update(gradient_norm=float(np.linalg.norm([float(g) for g in grad])), derivatives_not_none=len(grad))
     print(json.dumps({"num_products": len(prods), **counts, "paths": args.paths, "timeline_size": int(sc.simulation_timeline.numel()),
                       **shown,
                       "total_seconds": dt, "products_per_second": len(prods) / dt, "kernel_launches": B.launch_count() - l0,
